@@ -2,6 +2,7 @@
 """Benchmark on B200: the RGBA codec's encode + decode forward, its hot path, and the kernels' rooflines.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--legs forward,hotpath,config4,config5]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload "C2-forward" (BASELINE.json configs[1], per GPU): the full AutoEncoderRGB_Journal encode + decode forward
@@ -14,6 +15,8 @@ CUDA events around the module calls; `roofline` is the masked window-attention k
 Extra legs on the same JSON line: `hotpath` (round 1's workload: only the hot-path call sites, back to back),
 `config4` (attention microbench, 6 heads, 0-100 % masked), `config5` (training step of the codec on 256x256 crops with
 the NCCL gradient all-reduce).  Prints ONE JSON line (rank 0).
+--dump-outputs DIR writes what the last timed forward step returned (rank 0's shard) as DIR/<name>.npy, so that two
+builds run with the same arguments (same seeded inputs and weights) can be compared output for output.
 """
 from __future__ import annotations
 
@@ -240,6 +243,34 @@ def timed_steps(fn, steps, warmup, D: Dist):
     return D.max_ms(e0.elapsed_time(e1)) / steps, t0, time.time()
 
 
+# AutoEncoder.forward's return values (<package>/codec.py), in order
+FORWARD_OUTPUTS = ("x_hat", "mse", "bpp", "bpp_y", "bpp_z")
+DUMP_SAMPLE = 1 << 23            # elements kept of a larger output: 32 MB in float32, the whole dump stays under 64 MB
+DUMP_SEED = 0
+
+
+def dump_outputs(out_dir: str, names, tensors) -> None:
+    """DIR/<name>.npy per output, float64 kept, anything else as float32.  An output of more than DUMP_SAMPLE elements
+    is stored as flat[idx] with idx = sorted(randperm(numel, seed DUMP_SEED)[:DUMP_SAMPLE]): the same elements on every
+    run with the same arguments."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in zip(names, tensors, strict=True):
+        t = t.detach()
+        t = t if t.dtype == torch.float64 else t.float()
+        flat = t.reshape(-1)
+        if flat.numel() > DUMP_SAMPLE:
+            g = torch.Generator().manual_seed(DUMP_SEED)
+            idx = torch.randperm(flat.numel(), generator=g)[:DUMP_SAMPLE].sort().values
+            arr = flat[idx.to(flat.device)].cpu().numpy()
+        else:
+            arr = t.cpu().numpy()
+        total += arr.nbytes
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+    assert total <= 64 << 20, total
+
+
 # ------------------------------------------------------------------------------------------------ the codec workload
 def synthetic_rgba(batch: int, seed0: int) -> torch.Tensor:
     """(B, 4, H, W) in [0, 1]: smooth colour fields + noise, alpha = soft ellipse blobs; the colour planes are zero
@@ -310,7 +341,8 @@ def traffic_table():
         return json.load(f)
 
 
-def leg_forward(pkg, dev, rank, world, D, args, pk, tf32_convs=False, steps=None, want_e2e=True, sampler=None, library_convs=False):
+def leg_forward(pkg, dev, rank, world, D, args, pk, tf32_convs=False, steps=None, want_e2e=True, sampler=None, library_convs=False,
+                dump_dir=None):
     pkg.conv.USE_KERNEL = not library_convs
     torch.backends.cudnn.allow_tf32 = bool(tf32_convs)
     torch.backends.cuda.matmul.allow_tf32 = False
@@ -321,9 +353,12 @@ def leg_forward(pkg, dev, rank, world, D, args, pk, tf32_convs=False, steps=None
     rgba = rgba_host.to(dev)
     image, alpha = rgba[:, :3].contiguous(), rgba[:, 3:4].contiguous()
 
+    last = {}
+
     def step(img=image, a=alpha):
         me = net.EncMakeMask(a)                                  # trainRGB.py:283
-        return net(img, a, a, me[0], me[1], me[2], me[3])        # trainRGB.py:289 (reconmask = the alpha itself)
+        last["out"] = net(img, a, a, me[0], me[1], me[2], me[3])     # trainRGB.py:289 (reconmask = the alpha itself)
+        return last["out"]
 
     steps = steps or args.steps
     with torch.no_grad():
@@ -341,6 +376,8 @@ def leg_forward(pkg, dev, rank, world, D, args, pk, tf32_convs=False, steps=None
         timer.on = True
         ms_per_step, t0, t1 = timed_steps(step, steps, 0, D)
         timer.on = False
+        if dump_dir is not None and rank == 0:
+            dump_outputs(dump_dir, FORWARD_OUTPUTS, last["out"])
     clocks = sampler.stop(t0, t1) if sampler is not None else None
     per_op = timer.mean_ms()
     value = BATCH_PER_GPU * world / (ms_per_step * 1e-3)
@@ -618,7 +655,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-clocks", action="store_true", help="skip the nvidia-smi clock sampler (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed forward step as DIR/<name>.npy (a fixed, seeded sample of "
+                         "x_hat; rank 0's shard)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU forward (--impl ours)")
     if args.impl == "reference":
         return reference_arm(args)
     args.warmup = max(args.warmup, 3)
@@ -634,7 +676,8 @@ def main():
     pk = peaks()
 
     sampler = ClockSampler(local) if (rank == 0 and not args.no_clocks) else None      # needs ~0.5 s to start
-    fwd = leg_forward(pkg, dev, rank, world, D, args, pk, tf32_convs=False, want_e2e=not args.no_e2e, sampler=sampler)
+    fwd = leg_forward(pkg, dev, rank, world, D, args, pk, tf32_convs=False, want_e2e=not args.no_e2e, sampler=sampler,
+                      dump_dir=args.dump_outputs)
     extra = {}
     if "tf32" in legs:
         for key, tf32 in (("forward_library_convs_fp32", False), ("forward_library_convs_tf32", True)):

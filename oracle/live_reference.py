@@ -1,8 +1,9 @@
-"""Import the UNMODIFIED reference modules from /root/reference (build container only).
+"""Import the UNMODIFIED reference modules from the original project's source tree.
 
-TEST INFRASTRUCTURE ONLY.  /root/reference does not exist on the GPU box: nothing that runs
-there may call `load()`; use `available()` to gate.  No reference source is copied -- the
-modules are executed from where they lie, through the stand-in packages under shims/.
+TEST INFRASTRUCTURE ONLY.  The tree is not part of this repository: point MWA_REFERENCE_ROOT at a
+checkout of it to enable the tests that compare against it live; without it `available()` is False
+and they skip (tests/golden holds stored outputs of the same modules).  No reference source is
+copied -- the modules are executed from where they lie, through the stand-in packages under shims/.
 """
 from __future__ import annotations
 
@@ -10,12 +11,12 @@ import importlib
 import os
 import sys
 
-REFERENCE_ROOT = os.environ.get("MWA_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("MWA_REFERENCE_ROOT", "")
 _SHIMS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "shims")
 
 
 def available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "layers", "masked_win_attention.py"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(REFERENCE_ROOT, "layers", "masked_win_attention.py"))
 
 
 class _RefModules:
@@ -52,7 +53,7 @@ def load() -> _RefModules:
     if _cached is not None:
         return _cached
     if not available():
-        raise RuntimeError(f"reference tree not found at {REFERENCE_ROOT}")
+        raise RuntimeError(f"reference tree not found at MWA_REFERENCE_ROOT={REFERENCE_ROOT!r}")
     sys.dont_write_bytecode = True
     for p in (REFERENCE_ROOT, _SHIMS):
         if p not in sys.path:

@@ -30,7 +30,10 @@ def test_library_exports_every_declared_symbol(pkg):
 def test_library_has_no_torch_dependency(pkg):
     import subprocess
     out = subprocess.run(["ldd", pkg._abi.LIB_PATH], capture_output=True, text=True).stdout
-    assert "torch" not in out and "c10" not in out and "libcudart" not in out   # cudart linked statically
+    # dependency names and paths only: the load addresses ldd prints are random hex that may contain "c10"
+    deps = " ".join(tok for line in out.splitlines() for tok in line.split() if not tok.startswith("(0x"))
+    assert deps.strip()
+    assert "torch" not in deps and "c10" not in deps and "libcudart" not in deps   # cudart linked statically
 
 
 def test_status_strings_and_sizes(lib):
@@ -88,7 +91,7 @@ def test_constructor_contracts(pkg):
     torch.testing.assert_close(g.gamma ** 2 - g.pedestal, 0.1 * torch.eye(192), atol=1e-7, rtol=0)
 
 
-@pytest.mark.skipif(not live_reference.available(), reason="reference tree not present on this box")
+@pytest.mark.skipif(not live_reference.available(), reason="needs MWA_REFERENCE_ROOT: the original project's source tree")
 class TestAgainstReferenceSurface:
     def test_signatures_match(self, pkg):
         ref = live_reference.load()

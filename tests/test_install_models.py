@@ -1,5 +1,5 @@
-"""The reference's OWN model files import and build on top of the drop-in modules (build container only;
-runs in a subprocess because it re-binds the top-level `layers` package)."""
+"""The reference's OWN model files import and build on top of the drop-in modules (only where MWA_REFERENCE_ROOT names
+the original project's tree; runs in a subprocess because it re-binds the top-level `layers` package)."""
 import os
 import subprocess
 import sys
@@ -47,7 +47,7 @@ for k in keys: print(k)
 """
 
 
-@pytest.mark.skipif(not live_reference.available(), reason="reference tree not present on this box")
+@pytest.mark.skipif(not live_reference.available(), reason="needs MWA_REFERENCE_ROOT: the original project's source tree")
 def test_reference_models_build_on_dropins_with_identical_checkpoint_keys():
     fmt = dict(root=ROOT, ref=live_reference.REFERENCE_ROOT)
     env = dict(os.environ, PYTHONDONTWRITEBYTECODE="1")

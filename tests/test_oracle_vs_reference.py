@@ -1,11 +1,11 @@
-"""Oracle restatement vs the LIVE reference modules (only where /root/reference exists: the build container)."""
+"""Oracle restatement vs the LIVE reference modules (only where MWA_REFERENCE_ROOT names the original project's tree)."""
 import pytest
 import torch
 
 from oracle import live_reference
 from oracle import ref_ops as R
 
-pytestmark = pytest.mark.skipif(not live_reference.available(), reason="reference tree not present on this box")
+pytestmark = pytest.mark.skipif(not live_reference.available(), reason="needs MWA_REFERENCE_ROOT: the original project's source tree")
 
 
 @pytest.fixture(scope="module")
