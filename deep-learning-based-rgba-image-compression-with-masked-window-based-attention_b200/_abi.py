@@ -16,7 +16,7 @@ _PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_PKG_DIR, "libmwa_b200.so")
 
 MWA_OK = 0
-ALGO_AUTO, ALGO_SIMT, ALGO_TCGEN05, ALGO_TCGEN05_V1, ALGO_TCGEN05_FP16 = 0, 1, 2, 3, 4
+ALGO_AUTO, ALGO_SIMT, ALGO_TCGEN05 = 0, 1, 2
 ABI_VERSION = 1
 
 # name -> (restype, argtypes); mirrors include/mwa_b200.h one to one

@@ -65,20 +65,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
     while (!mbar_try_wait(bar, parity)) {
     }
 }
-// wait with an explicit hardware suspend hint: the warp sleeps until the phase completes (or the hint expires)
-// instead of re-issuing the probe -- keeps waiting warps out of the issue slots of the warp that does the work
-__device__ __forceinline__ void mbar_wait_sleep(uint64_t* bar, uint32_t parity) {
-    uint32_t ok;
-    do {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}\n"
-            : "=r"(ok)
-            : "r"(smem_u32(bar)), "r"(parity), "r"(0x989680u)
-            : "memory");
-    } while (!ok);
-}
 
 // generic-proxy smem writes -> visible to the async proxy (UMMA operand reads, bulk copies)
 __device__ __forceinline__ void fence_proxy_async_smem() {

@@ -1,27 +1,12 @@
 // Masked window attention: parameter preparation and the general-shape SIMT forward kernel.
 // Reference semantics: layers/masked_win_attention.py:169-251 (block), :96-131 (window attention),
 // :35-47 (keep predicate), :194-216 (SW-MSA region mask); layers/win_attention.py:153-207 (alpha == NULL).
-// The tcgen05 forward for the model's configurations lives in mwa_tc.cu.
+// The forwards for the model's configurations live in mwa_sp.cu (8x8 windows, C = 192) and mwa_small.cu (4x4, C = 80).
 #include "common.cuh"
 #include "params.cuh"
 #include "status.cuh"
 
 namespace b200 {
-
-int mwa_forward_tc(const float* x, const float* alpha, float* out, const void* params, int B, int C, int H, int W,
-                   int heads, int ws, int shift, int channels_last, int32_t* kept_count, void* workspace,
-                   int64_t workspace_bytes, cudaStream_t st);                                                // mwa_tc.cu
-int64_t mwa_tc_workspace_bytes(int64_t nwin);
-void mwa_tc_set_timing_buffer(void* p);
-bool mwa_tc_supported(int C, int heads, int ws, int H, int W, int shift, int channels_last);
-void mwa_tc_prepare_images(const float* qkv_w, const float* qkv_b, const float* proj_w, const float* proj_b, int C,
-                           int heads, int ws, float scale, uint8_t* blk, cudaStream_t st);                    // mwa_tc.cu
-
-int mwa_forward_ws(const float* x, const float* alpha, float* out, const void* params, int B, int C, int H, int W,
-                   int heads, int ws, int shift, int32_t* kept_count, void* workspace, int64_t workspace_bytes,
-                   cudaStream_t st);                                                                          // mwa_ws.cu
-bool mwa_ws_supported(int C, int heads, int ws, int channels_last);
-void mwa_ws_set_timing_buffer(void* p);
 
 int mwa_forward_sp(const float* x, const float* alpha, float* out, const void* params, int B, int C, int H, int W,
                    int heads, int ws, int shift, int32_t* kept_count, void* workspace, int64_t workspace_bytes,
@@ -296,26 +281,19 @@ int mwa_prepare(const float* qkv_w, const float* qkv_b, const float* proj_w, con
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     uint8_t* blk = static_cast<uint8_t*>(params);
     mwa_prepare_kernel<<<148, 256, 0, st>>>(qkv_w, qkv_b, proj_w, proj_b, bias_table, C, heads, ws, scale, blk);
-    int rc = check_launch("mwa_prepare");
-    if (rc != MWA_OK) return rc;
-    mwa_tc_prepare_images(qkv_w, qkv_b, proj_w, proj_b, C, heads, ws, scale, blk, st);
-    rc = check_launch("mwa_prepare(images)");
+    const int rc = check_launch("mwa_prepare");
     if (rc != MWA_OK) return rc;
     mwa_sp_prepare_images(qkv_w, qkv_b, proj_w, proj_b, bias_table, C, heads, ws, scale, blk, st);
     return check_launch("mwa_prepare(split-precision images)");
 }
 
-void mwa_debug_set_timing_buffer(void* device_u64x4096) {
-    mwa_tc_set_timing_buffer(device_u64x4096);
-    mwa_ws_set_timing_buffer(device_u64x4096);
-    mwa_sp_set_timing_buffer(device_u64x4096);
-}
+void mwa_debug_set_timing_buffer(void* device_u64x8192) { mwa_sp_set_timing_buffer(device_u64x8192); }
 
 int64_t mwa_workspace_bytes(int B, int H, int W, int ws) {
     if (B < 0 || H <= 0 || W <= 0 || ws <= 0) return MWA_ERR_INVALID;
     const int64_t nwin = int64_t(B) * (H / ws) * (W / ws);
-    const int64_t a = mwa_tc_workspace_bytes(nwin), b = mwa_sp_workspace_bytes(nwin), c = mwa_small_workspace_bytes(nwin);
-    return a > b ? (a > c ? a : c) : (b > c ? b : c);
+    const int64_t a = mwa_sp_workspace_bytes(nwin), b = mwa_small_workspace_bytes(nwin);
+    return a > b ? a : b;
 }
 
 int mwa_fast_path_needs_nchw(int C, int heads, int ws) {
@@ -328,17 +306,16 @@ int mwa_forward(const float* x, const float* alpha, float* out, const void* para
     if (B < 0 || C <= 0 || H <= 0 || W <= 0 || heads <= 0 || ws <= 0 || C % heads != 0) return MWA_ERR_INVALID;
     if (shift < 0 || shift >= ws) return MWA_ERR_INVALID;
     if (H % ws != 0 || W % ws != 0) return MWA_ERR_INVALID;
+    if (algo != MWA_ALGO_AUTO && algo != MWA_ALGO_SIMT && algo != MWA_ALGO_TCGEN05) return MWA_ERR_INVALID;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (kept_count) MWA_TRY_CUDA(cudaMemsetAsync(kept_count, 0, sizeof(int32_t), st), "mwa_forward(memset)");
     if (B == 0) return MWA_OK;                              // empty batch: x / out may be null
     if (!x || !out || !params) return MWA_ERR_INVALID;
-    const bool tc_ok = mwa_tc_supported(C, heads, ws, H, W, shift, channels_last);
     // MWA_ALGO_AUTO is fp32-faithful on every shape (the reference's arithmetic is fp32 end to end):
     //   8x8 windows, C = 192: split-precision tcgen05 kernel (every operand fp16 hi + lo, three passes);
     //   4x4 windows, C = 80:  plain fp32 kernel for small windows;
     //   anything else:        the general fp32 SIMT kernel.
-    // The single-pass fp16 tensor-core kernels (faster, ~1e-4 .. 3e-4 absolute error at random init) are opt-in:
-    // MWA_ALGO_TCGEN05_FP16 / MWA_ALGO_TCGEN05_V1, and MWA_ALGO_TCGEN05 where no split-precision kernel covers the shape.
+    // MWA_ALGO_TCGEN05 asks for the split-precision kernel and fails where it does not cover the shape.
     if ((algo == MWA_ALGO_AUTO || algo == MWA_ALGO_TCGEN05) && mwa_sp_supported(C, heads, ws, H, W, channels_last)) {
         if (!aligned16(x) || !aligned16(out)) return MWA_ERR_ALIGNMENT;
         return mwa_forward_sp(x, alpha, out, params, B, C, H, W, heads, ws, shift, kept_count, workspace, workspace_bytes, st);
@@ -348,16 +325,7 @@ int mwa_forward(const float* x, const float* alpha, float* out, const void* para
         return mwa_forward_small(x, alpha, out, params, B, C, H, W, heads, ws, shift, kept_count, workspace, workspace_bytes,
                                  st);
     }
-    if (algo == MWA_ALGO_TCGEN05 || algo == MWA_ALGO_TCGEN05_V1 || algo == MWA_ALGO_TCGEN05_FP16) {
-        if (!tc_ok) return MWA_ERR_UNSUPPORTED;
-        if (!aligned16(x) || !aligned16(out)) return MWA_ERR_ALIGNMENT;
-        // warp-specialised pipeline where it covers the layout, else the phase-serial v1 kernel
-        if (algo != MWA_ALGO_TCGEN05_V1 && mwa_ws_supported(C, heads, ws, channels_last))
-            return mwa_forward_ws(x, alpha, out, params, B, C, H, W, heads, ws, shift, kept_count, workspace,
-                                  workspace_bytes, st);
-        return mwa_forward_tc(x, alpha, out, params, B, C, H, W, heads, ws, shift, channels_last, kept_count, workspace,
-                              workspace_bytes, st);
-    }
+    if (algo == MWA_ALGO_TCGEN05) return MWA_ERR_UNSUPPORTED;
     const int N = ws * ws;
     if (N > 64) return MWA_ERR_UNSUPPORTED;
     const int64_t smem = 4ll * (int64_t(N) * C + int64_t(N) * (3 * C + 1) + int64_t(N) * (N + 1));

@@ -1,14 +1,58 @@
-// Kept / dropped window lists and the copy of the dropped windows, shared by the kernels that work from an ordered list
-// of kept windows (csrc/mwa_sp.cu: 8x8 windows on tcgen05; csrc/mwa_small.cu: 4x4 windows in fp32).
-// Reference semantics: layers/masked_win_attention.py:35-47 (keep predicate), :237-249 (dropped windows contribute zeros,
-// i.e. the block is the identity there).
+// Window geometry, keep flags, kept / dropped window lists, the copy of the dropped windows and the host front end that
+// launches them, shared by the kernels that work from an ordered list of kept windows (csrc/mwa_sp.cu: 8x8 windows on
+// tcgen05; csrc/mwa_small.cu: 4x4 windows in fp32).
+// Reference semantics: layers/masked_win_attention.py:6-47 (partition, keep predicate), :237-249 (dropped windows
+// contribute zeros, i.e. the block is the identity there).
 #pragma once
-#include "mwa_tc_shared.cuh"
+#include "common.cuh"
+#include "params.cuh"
+#include "status.cuh"
 
 namespace b200 {
 namespace {
 
+constexpr float kNegMask = -100.0f;                 // layers/masked_win_attention.py:214
+
+struct Geom {
+    int B, H, W, shift, nwx, nwy, channels_last;
+};
+
+__device__ __forceinline__ void window_coords(const Geom& g, int win, int& b, int& wy, int& wx) {
+    b = win / (g.nwy * g.nwx);
+    const int r = win - b * g.nwy * g.nwx;
+    wy = r / g.nwx;
+    wx = r - wy * g.nwx;
+}
+// token t of window (wy, wx): original (un-shifted) pixel
+template <int WS>
+__device__ __forceinline__ void token_pixel(const Geom& g, int wy, int wx, int t, int& y, int& x) {
+    y = wy * WS + t / WS + g.shift;
+    if (y >= g.H) y -= g.H;
+    x = wx * WS + t % WS + g.shift;
+    if (x >= g.W) x -= g.W;
+}
+
 // ------------------------------------------------------------------------------------------------ scan / compaction
+// one warp per window: keep flag = (sum of the window's alpha != 0)
+template <int WS>
+__global__ void __launch_bounds__(256)
+mwa_scan_kernel(const float* __restrict__ alpha, Geom g, int nwin, uint8_t* __restrict__ flags) {
+    constexpr int NTOK = WS * WS;
+    const int win = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (win >= nwin) return;
+    int b, wy, wx;
+    window_coords(g, win, b, wy, wx);
+    float a = 0.f;
+    for (int t = lane; t < NTOK; t += 32) {
+        int y, xx;
+        token_pixel<WS>(g, wy, wx, t, y, xx);
+        a += __ldg(alpha + (int64_t(b) * g.H + y) * g.W + xx);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+    if (lane == 0) flags[win] = a != 0.f;
+}
+
 struct ListWs {             // workspace layout: counts (kept, dropped), keep flags, kept list, dropped list
     int64_t count, flags, list, dlist, total;
     __host__ __device__ explicit ListWs(int64_t nwin) {
@@ -139,6 +183,46 @@ mwa_copy_dropped_kernel(const float* __restrict__ x, float* __restrict__ out, Ge
             }
         }
     }
+}
+
+// ------------------------------------------------------------------------------------------------ host front end
+// Everything a list-based forward does around its main kernel: checks the window count and the workspace, builds the
+// keep flags and the ordered kept / dropped lists in the workspace (alpha == nullptr keeps every window), copies the
+// dropped windows x -> out, then calls launch(nwin, list, count) for the main kernel (count[0] = kept windows, on the
+// device) and finally copies the kept count to kept_count (may be nullptr).
+template <int WS, class Launch>
+int mwa_forward_lists(const float* x, const float* alpha, float* out, const Geom& geo, int C, int32_t* kept_count,
+                      void* workspace, int64_t workspace_bytes, cudaStream_t st, Launch launch) {
+    const int64_t nwin64 = int64_t(geo.B) * geo.nwx * geo.nwy;
+    if (nwin64 > 0x3fffffffll) return MWA_ERR_UNSUPPORTED;
+    const int nwin = static_cast<int>(nwin64);
+    const ListWs ws(nwin);
+    if (!workspace || workspace_bytes < ws.total) return MWA_ERR_WORKSPACE;
+    if (!aligned16(workspace)) return MWA_ERR_ALIGNMENT;
+    uint8_t* wsp = static_cast<uint8_t*>(workspace);
+    int32_t* count = reinterpret_cast<int32_t*>(wsp + ws.count);
+    uint8_t* flags = wsp + ws.flags;
+    int32_t* list = reinterpret_cast<int32_t*>(wsp + ws.list);
+    int32_t* dlist = reinterpret_cast<int32_t*>(wsp + ws.dlist);
+    int rc;
+    if (alpha != nullptr) {
+        mwa_scan_kernel<WS><<<(nwin + 7) / 8, 256, 0, st>>>(alpha, geo, nwin, flags);
+        rc = check_launch("mwa_forward(scan)");
+        if (rc != MWA_OK) return rc;
+    }
+    mwa_list_compact_kernel<<<1, 1024, 0, st>>>(alpha ? flags : nullptr, nwin, list, dlist, count);
+    rc = check_launch("mwa_forward(compact)");
+    if (rc != MWA_OK) return rc;
+    if (alpha != nullptr && out != x) {
+        mwa_copy_dropped_kernel<WS><<<kNumSMs * 8, 256, 0, st>>>(x, out, geo, C, flags, dlist, count);
+        rc = check_launch("mwa_forward(copy dropped)");
+        if (rc != MWA_OK) return rc;
+    }
+    rc = launch(nwin, list, count);
+    if (rc != MWA_OK) return rc;
+    if (kept_count)
+        MWA_TRY_CUDA(cudaMemcpyAsync(kept_count, count, sizeof(int32_t), cudaMemcpyDeviceToDevice, st), "mwa_forward(kept_count)");
+    return MWA_OK;
 }
 
 }  // namespace

@@ -13,7 +13,6 @@
 //            (+ SW-MSA region mask), softmax, P V -- no shuffles, no barriers inside
 //   proj     [64 x C] x [C x C]: thread = 4 tokens x C/16 outputs, + bias + residual, float2 stores (a window row)
 // Dropped windows are copied through by mwa_copy_dropped_kernel (only the dropped ones).
-#include "mwa_tc_shared.cuh"
 #include "mwa_lists.cuh"
 
 namespace b200 {
@@ -277,42 +276,16 @@ template <class CF>
 int launch_small(const float* x, const float* alpha, float* out, const uint8_t* params, int B, int H, int W, int shift,
                  int32_t* kept_count, void* workspace, int64_t workspace_bytes, cudaStream_t st) {
     const Geom geo{B, H, W, shift, W / CF::WS, H / CF::WS, 0};
-    const int64_t nwin64 = int64_t(B) * geo.nwx * geo.nwy;
-    if (nwin64 > 0x3fffffffll) return MWA_ERR_UNSUPPORTED;
-    const int nwin = static_cast<int>(nwin64);
-    const ListWs ws(nwin);
-    if (!workspace || workspace_bytes < ws.total) return MWA_ERR_WORKSPACE;
-    if (!aligned16(workspace)) return MWA_ERR_ALIGNMENT;
-    uint8_t* wsp = static_cast<uint8_t*>(workspace);
-    int32_t* count = reinterpret_cast<int32_t*>(wsp + ws.count);
-    uint8_t* flags = wsp + ws.flags;
-    int32_t* list = reinterpret_cast<int32_t*>(wsp + ws.list);
-    int32_t* dlist = reinterpret_cast<int32_t*>(wsp + ws.dlist);
-    int rc;
-    if (alpha != nullptr) {
-        mwa_scan_kernel<CF::WS, 1><<<(nwin + 7) / 8, 256, 0, st>>>(x, alpha, out, geo, CF::C, nwin, flags, 0);
-        rc = check_launch("mwa_forward(scan)");
-        if (rc != MWA_OK) return rc;
-    }
-    mwa_list_compact_kernel<<<1, 1024, 0, st>>>(alpha ? flags : nullptr, nwin, list, dlist, count);
-    rc = check_launch("mwa_forward(compact)");
-    if (rc != MWA_OK) return rc;
-    if (alpha != nullptr && out != x) {
-        mwa_copy_dropped_kernel<CF::WS><<<kNumSMs * 8, 256, 0, st>>>(x, out, geo, CF::C, flags, dlist, count);
-        rc = check_launch("mwa_forward(copy dropped)");
-        if (rc != MWA_OK) return rc;
-    }
-    const int smem = CF::total * 4;
-    MWA_TRY_CUDA(cudaFuncSetAttribute(mwa_small_kernel<CF>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem),
-                 "mwa_forward(small attr)");
-    const int max_groups = (nwin + CF::GW - 1) / CF::GW;
-    const int grid = max_groups < kNumSMs ? max_groups : kNumSMs;
-    mwa_small_kernel<CF><<<grid, 256, smem, st>>>(x, out, params, list, count, geo);
-    rc = check_launch("mwa_forward(fp32 small windows)");
-    if (rc != MWA_OK) return rc;
-    if (kept_count)
-        MWA_TRY_CUDA(cudaMemcpyAsync(kept_count, count, sizeof(int32_t), cudaMemcpyDeviceToDevice, st), "mwa_forward(kept_count)");
-    return MWA_OK;
+    return mwa_forward_lists<CF::WS>(x, alpha, out, geo, CF::C, kept_count, workspace, workspace_bytes, st,
+                                     [&](int nwin, const int32_t* list, const int32_t* count) -> int {
+        const int smem = CF::total * 4;
+        MWA_TRY_CUDA(cudaFuncSetAttribute(mwa_small_kernel<CF>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem),
+                     "mwa_forward(small attr)");
+        const int max_groups = (nwin + CF::GW - 1) / CF::GW;
+        const int grid = max_groups < kNumSMs ? max_groups : kNumSMs;
+        mwa_small_kernel<CF><<<grid, 256, smem, st>>>(x, out, params, list, count, geo);
+        return check_launch("mwa_forward(fp32 small windows)");
+    });
 }
 
 }  // namespace

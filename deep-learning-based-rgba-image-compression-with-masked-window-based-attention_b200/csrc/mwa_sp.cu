@@ -1,6 +1,6 @@
 // Fused masked window attention forward in SPLIT PRECISION (fp32-faithful results on the tensor cores), sm_100a only.
 // Reference semantics: layers/masked_win_attention.py:169-251 (block) and :96-131 (window attention), whose arithmetic
-// is fp32 end to end.  A single fp16 pass per contraction (csrc/mwa_ws.cu) misses the 1e-3 rel / 1e-4 abs contract on
+// is fp32 end to end.  A single fp16 pass per contraction misses the 1e-3 rel / 1e-4 abs contract on
 // ~0.1 % of the outputs at random init and by far more on weights with large logits; tools/precision_study.py shows
 // which operand roundings cost what.  Here EVERY operand of EVERY contraction (x, Wqkv, q, k, v, P, O, Wproj) is carried
 // as fp16 hi + lo and contracted in three passes (hi*hi + lo*hi + hi*lo, fp32 accumulation in TMEM): ~2^-21 relative
@@ -34,7 +34,6 @@
 // Dropped windows are copied through by a separate small kernel (only the dropped ones).
 #include <cstring>
 #include <cuda.h>          // CUtensorMap (type only: the encoder is fetched through cudaGetDriverEntryPoint)
-#include "mwa_tc_shared.cuh"
 #include "mwa_lists.cuh"
 
 // bring-up switches (tools/build_variants.py)
@@ -54,6 +53,7 @@ constexpr int kSpMma = 0, kSpFeed = 1, kSpTma0 = 2;
 constexpr int kSpPe0 = 4, kSpNumPe = 8, kSpSm0 = 12, kSpNumSm = 8, kSpDr0 = 20;
 // register pool of the CTA = 24 warps x 80 (launch bound); per SM sub-partition 56 + 2 x 88 + 2 x 80 + 88 = 480 = 6 x 80
 constexpr int kSpRegsCtl = 56, kSpRegsPe = 88, kSpRegsSm = 80, kSpRegsDr = 88;
+constexpr float kLog2e = 1.4426950408889634f;
 constexpr float kNegMaskL2 = kNegMask * kLog2e;
 
 template <int HEADS_>
@@ -109,6 +109,11 @@ struct SpParams {
     static constexpr int64_t i16 = tbl + (int64_t(CF::HEADS) * CF::TBL * 4 + 1023) / 1024 * 1024;
     static constexpr int64_t total = i16 + 2048;
 };
+
+__global__ void zero16_kernel(uint4* p, int64_t n16) {
+    for (int64_t i = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; i < n16; i += int64_t(gridDim.x) * blockDim.x)
+        p[i] = make_uint4(0, 0, 0, 0);
+}
 
 __device__ __forceinline__ uint16_t f16_bits(float v) { return __half_as_ushort(__float2half_rn(v)); }
 __device__ __forceinline__ float f16_round(float v) { return __half2float(__float2half_rn(v)); }
@@ -173,6 +178,14 @@ __device__ __forceinline__ void split_f16x2(float a, float b, uint32_t& hi, uint
     const float2 hf = __half22float2(h);
     hi = *reinterpret_cast<const uint32_t*>(&h);
     lo = pack_f16x2(a - hf.x, b - hf.y);
+}
+__device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
+    asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
+}
+__device__ __forceinline__ float ex2(float v) {
+    float r;
+    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(v));
+    return r;
 }
 __device__ __forceinline__ float max3(float a, float b, float c) {
     float r;
@@ -885,52 +898,26 @@ template <class CF>
 int launch_sp(const float* x, const float* alpha, float* out, const uint8_t* sp, int B, int H, int W, int shift,
               int32_t* kept_count, void* workspace, int64_t workspace_bytes, cudaStream_t st) {
     const Geom geo{B, H, W, shift, W / CF::WS, H / CF::WS, 0};
-    const int64_t nwin64 = int64_t(B) * geo.nwx * geo.nwy;
-    if (nwin64 > 0x3fffffffll) return MWA_ERR_UNSUPPORTED;
-    const int nwin = static_cast<int>(nwin64);
-    const ListWs ws(nwin);
-    if (!workspace || workspace_bytes < ws.total) return MWA_ERR_WORKSPACE;
-    if (!aligned16(workspace)) return MWA_ERR_ALIGNMENT;
-    uint8_t* wsp = static_cast<uint8_t*>(workspace);
-    int32_t* count = reinterpret_cast<int32_t*>(wsp + ws.count);
-    uint8_t* flags = wsp + ws.flags;
-    int32_t* list = reinterpret_cast<int32_t*>(wsp + ws.list);
-    int32_t* dlist = reinterpret_cast<int32_t*>(wsp + ws.dlist);
-    int rc;
-    if (alpha != nullptr) {
-        mwa_scan_kernel<CF::WS, 1><<<(nwin + 7) / 8, 256, 0, st>>>(x, alpha, out, geo, CF::C, nwin, flags, 0);
-        rc = check_launch("mwa_forward(scan)");
+    return mwa_forward_lists<CF::WS>(x, alpha, out, geo, CF::C, kept_count, workspace, workspace_bytes, st,
+                                     [&](int nwin, const int32_t* list, const int32_t* count) -> int {
+        CUtensorMap x_map;
+        memset(&x_map, 0, sizeof(x_map));
+        const int rc = sp_window_box_map(x, B, CF::C, H, W, &x_map);
         if (rc != MWA_OK) return rc;
-    }
-    mwa_list_compact_kernel<<<1, 1024, 0, st>>>(alpha ? flags : nullptr, nwin, list, dlist, count);
-    rc = check_launch("mwa_forward(compact)");
-    if (rc != MWA_OK) return rc;
-    if (alpha != nullptr && out != x) {
-        mwa_copy_dropped_kernel<CF::WS><<<kNumSMs * 8, 256, 0, st>>>(x, out, geo, CF::C, flags, dlist, count);
-        rc = check_launch("mwa_forward(copy dropped)");
-        if (rc != MWA_OK) return rc;
-    }
-    CUtensorMap x_map;
-    memset(&x_map, 0, sizeof(x_map));
-    rc = sp_window_box_map(x, B, CF::C, H, W, &x_map);
-    if (rc != MWA_OK) return rc;
-    const int smem = CF::oTotal;
-    const int max_tiles = (nwin + 1) / 2;
-    const int grid = max_tiles < kNumSMs ? max_tiles : kNumSMs;
-    if (g_sp_timing != nullptr) {
-        MWA_TRY_CUDA(cudaFuncSetAttribute(mwa_sp_kernel<CF, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem),
-                     "mwa_forward(sp attr)");
-        mwa_sp_kernel<CF, true><<<grid, kSpThreads, smem, st>>>(x, out, sp, list, count, geo, g_sp_timing, x_map);
-    } else {
-        MWA_TRY_CUDA(cudaFuncSetAttribute(mwa_sp_kernel<CF, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem),
-                     "mwa_forward(sp attr)");
-        mwa_sp_kernel<CF, false><<<grid, kSpThreads, smem, st>>>(x, out, sp, list, count, geo, nullptr, x_map);
-    }
-    rc = check_launch("mwa_forward(tcgen05 split precision)");
-    if (rc != MWA_OK) return rc;
-    if (kept_count)
-        MWA_TRY_CUDA(cudaMemcpyAsync(kept_count, count, sizeof(int32_t), cudaMemcpyDeviceToDevice, st), "mwa_forward(kept_count)");
-    return MWA_OK;
+        const int smem = CF::oTotal;
+        const int max_tiles = (nwin + 1) / 2;
+        const int grid = max_tiles < kNumSMs ? max_tiles : kNumSMs;
+        if (g_sp_timing != nullptr) {
+            MWA_TRY_CUDA(cudaFuncSetAttribute(mwa_sp_kernel<CF, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem),
+                         "mwa_forward(sp attr)");
+            mwa_sp_kernel<CF, true><<<grid, kSpThreads, smem, st>>>(x, out, sp, list, count, geo, g_sp_timing, x_map);
+        } else {
+            MWA_TRY_CUDA(cudaFuncSetAttribute(mwa_sp_kernel<CF, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem),
+                         "mwa_forward(sp attr)");
+            mwa_sp_kernel<CF, false><<<grid, kSpThreads, smem, st>>>(x, out, sp, list, count, geo, nullptr, x_map);
+        }
+        return check_launch("mwa_forward(tcgen05 split precision)");
+    });
 }
 
 }  // namespace

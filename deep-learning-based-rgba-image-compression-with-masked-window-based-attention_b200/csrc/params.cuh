@@ -35,17 +35,6 @@ struct GdnParamLayout {
 };
 
 // ---------------------------------------------------------------- masked window attention
-// size of the tcgen05 section (fp16 weight operand images per head group + padded-order qkv bias + the projection bias
-// with the v bias folded in); mirrors Cfg<> /
-// TcParams<> in mwa_tc.cu.  0 when the head geometry has no tcgen05 mapping.
-__host__ __device__ inline int64_t mwa_tc_section_bytes(int C, int heads) {
-    const int d = C / heads, dpad = (d + 15) / 16 * 16;
-    if (dpad > 64 || 64 % dpad != 0 || heads % (64 / dpad) != 0 || C % 16 != 0) return 0;
-    const int64_t hpg = 64 / dpad, ng = heads / hpg, kb = (C + 63) / 64;
-    const int64_t nqkv = (3 * hpg * d + 15) / 16 * 16;
-    return ng * (kb * nqkv * 128 + int64_t(C) * 128) + ng * nqkv * 4 + int64_t(C) * 4;
-}
-
 // size of the split-precision section (csrc/mwa_sp.cu, layout: SpParams<> there): per head the fp16 hi and lo
 // K-major SW128 slabs of Wq|Wk|Wv per 64-channel K block as ring-slot sized elements, per head and output half the
 // [hi | lo] slab of Wproj, the scaled q bias, the projection bias with the v bias folded in, the relative-position
@@ -57,21 +46,17 @@ __host__ __device__ inline int64_t mwa_sp_section_bytes(int C, int heads, int ws
 }
 
 struct MwaParamLayout {
-    int C, heads, ws, N, d, dpad, kblocks;
+    int C, heads, ws, N, d;
     int64_t header;     // float[4]: scale, -, -, -
     int64_t wqkvT;      // fp32 [C][3C]   qkv.weight transposed  ([in][out])
     int64_t bqkv;       // fp32 [3C]      (zeros when qkv_bias=False)
     int64_t wprojT;     // fp32 [C][C]    proj.weight transposed
     int64_t bproj;      // fp32 [C]
     int64_t bias;       // fp32 [heads][N][N]   expanded relative position bias
-    int64_t img_wqkv;   // tcgen05 section (layout: TcParams<> in mwa_tc.cu): per head group the fp16 K-major SW128
-                        // B-operand slabs of Wq|Wk|Wv (rows head-padded to 16/32, q rows pre-scaled) and of Wproj,
-                        // followed by the qkv bias in the same padded order
     int64_t img_sp;     // split-precision section (layout: SpParams<> in mwa_sp.cu)
     int64_t total;
     __host__ __device__ MwaParamLayout(int C_, int heads_, int ws_)
-        : C(C_), heads(heads_), ws(ws_), N(ws_ * ws_), d(C_ / heads_), dpad(int(align_up(C_ / heads_, 16))),
-          kblocks((C_ + 63) / 64) {
+        : C(C_), heads(heads_), ws(ws_), N(ws_ * ws_), d(C_ / heads_) {
         int64_t o = 0;
         header = o;    o = align_up(o + 16, 1024);
         wqkvT = o;     o = align_up(o + 4ll * C * 3 * C, 1024);
@@ -79,7 +64,6 @@ struct MwaParamLayout {
         wprojT = o;    o = align_up(o + 4ll * C * C, 1024);
         bproj = o;     o = align_up(o + 4ll * C, 1024);
         bias = o;      o = align_up(o + 4ll * heads * N * N, 1024);
-        img_wqkv = o;  o = align_up(o + mwa_tc_section_bytes(C, heads), 1024);
         img_sp = o;    o = align_up(o + mwa_sp_section_bytes(C, heads, ws), 1024);
         total = o;
     }

@@ -53,7 +53,7 @@ class WindowAttentionFunction(Function):
         channels_last = (not x.is_contiguous()) and x.is_contiguous(memory_format=torch.channels_last)
         # The fp32-faithful fast kernels read NCHW.  A channels-last input goes through them too (one transposing copy
         # each way: far cheaper than the general SIMT kernel, which is what the C ABI falls back to for NHWC); the output
-        # keeps the input's memory format, as torch ops do.  Only the opt-in fp16 kernels consume NHWC in place.
+        # keeps the input's memory format, as torch ops do.  Only the general SIMT kernel consumes NHWC in place.
         relayout = channels_last and algo in (_abi.ALGO_AUTO, _abi.ALGO_TCGEN05) and \
             bool(lib.mwa_fast_path_needs_nchw(C, attn_mod.num_heads, ws))
         if relayout or not channels_last:

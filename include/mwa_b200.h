@@ -45,10 +45,9 @@ enum {
  *   C = 192, 8 x 8 windows, 6 or 8 heads, NCHW   split-precision tcgen05 kernel (every operand fp16 hi + lo, 3 MMA passes)
  *   C = 80, 4 x 4 windows, 8 heads, NCHW         plain fp32 kernel for small windows
  *   anything else                                general fp32 SIMT kernel (also what SIMT forces)
- * The single-pass fp16 tensor-core kernels of round 1 (faster, ~1e-4 .. 3e-4 absolute error at random init) are opt-in:
- * TCGEN05_FP16, TCGEN05_V1 (phase-serial first generation, kept for A/B measurements) and TCGEN05 on the shapes that
- * have no split-precision kernel. */
-enum { MWA_ALGO_AUTO = 0, MWA_ALGO_SIMT = 1, MWA_ALGO_TCGEN05 = 2, MWA_ALGO_TCGEN05_V1 = 3, MWA_ALGO_TCGEN05_FP16 = 4 };
+ * TCGEN05 forces the tensor-core kernel: the split-precision kernel for attention, the tcgen05 kernel for GDN;
+ * MWA_ERR_UNSUPPORTED where it does not cover the shape.  Any other value is MWA_ERR_INVALID. */
+enum { MWA_ALGO_AUTO = 0, MWA_ALGO_SIMT = 1, MWA_ALGO_TCGEN05 = 2 };
 
 MWA_API int mwa_b200_abi_version(void);
 MWA_API const char* mwa_b200_status_string(int status);
@@ -114,16 +113,18 @@ MWA_API int gdn_bwd_finalize(const float* dn, const float* dgamma_eff, const flo
  *
  * mwa_prepare : packs qkv.weight (3C,C), qkv.bias (3C) or NULL, proj.weight (C,C), proj.bias (C),
  *               relative_position_bias_table ((2ws-1)^2, heads) into `params`: fp32 transposes, the
- *               expanded (heads, N, N) bias (layers/masked_win_attention.py:109-112) and fp16 UMMA images.
+ *               expanded (heads, N, N) bias (layers/masked_win_attention.py:109-112) and, where the split-precision
+ *               kernel covers the shape, its fp16 hi / lo UMMA images.
  * mwa_forward : out = x + scatter(window_attention(kept windows of roll(x, -shift)))  rolled back;
  *               a window is kept iff the sum of its (shifted) alpha is != 0; alpha == NULL keeps all.
  *               x/out logical shape (B, C, H, W), alpha (B, 1, H, W); H % ws == 0 and W % ws == 0
  *               (else MWA_ERR_INVALID, the reference raises in .view); 0 <= shift < ws.
  *               `kept_count` (optional device int32, may be NULL) receives the number of kept windows.
  *               `workspace` (>= mwa_workspace_bytes(B, H, W, ws) bytes, 16-byte aligned, device) holds the keep flags
- *               and the compacted list of kept windows of the tcgen05 path; contents are scratch.
+ *               and the ordered lists of kept and dropped windows of the split-precision and small-window kernels;
+ *               contents are scratch.
  * Supported: ws*ws <= 64 tokens, C % heads == 0, shared memory footprint <= 227 KB (SIMT: C <= 192 at ws 8);
- *            tcgen05: (C, heads, ws) in {(192, 8, 8), (192, 6, 8), (80, 8, 4)}.
+ *            tcgen05 (split precision): (C, heads, ws) in {(192, 8, 8), (192, 6, 8)}, NCHW.
  * ------------------------------------------------------------------------------------------------ */
 MWA_API int64_t mwa_param_bytes(int C, int heads, int ws);
 MWA_API int mwa_prepare(const float* qkv_w, const float* qkv_b, const float* proj_w, const float* proj_b,
@@ -133,10 +134,10 @@ MWA_API int64_t mwa_workspace_bytes(int B, int H, int W, int ws);
 /* 1 when MWA_ALGO_AUTO has a fast fp32-faithful kernel for this configuration that reads NCHW only (the host layer then
  * hands a channels-last tensor over as NCHW instead of letting it fall to the general SIMT kernel), else 0 */
 MWA_API int mwa_fast_path_needs_nchw(int C, int heads, int ws);
-/* development aid: device buffer of 4096 uint64 that the tcgen05 attention kernels fill with clock64() totals
- * ([0,32): per-stage totals of CTA 0; [64,320): cycles per CTA; [320,576): tiles per CTA).  NULL switches it off
- * (the default). */
-MWA_API void mwa_debug_set_timing_buffer(void* device_u64x4096);
+/* development aid: device buffer of 8192 uint64 that the split-precision attention kernel fills with clock64() totals
+ * ([64,320): cycles per CTA; [320,576): tiles per CTA; [1024,5120): event trace of CTA 0, 1024 per role).  NULL switches
+ * it off (the default). */
+MWA_API void mwa_debug_set_timing_buffer(void* device_u64x8192);
 MWA_API int mwa_forward(const float* x, const float* alpha, float* out, const void* params, int B, int C, int H, int W,
                 int heads, int ws, int shift, int channels_last, int algo, int32_t* kept_count, void* workspace,
                 int64_t workspace_bytes, void* stream);

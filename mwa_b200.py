@@ -54,5 +54,4 @@ masked_psnr = metrics.masked_psnr
 HostPipeline = pipeline.HostPipeline
 invalidate_param_blocks = _params.invalidate_param_blocks
 MwaB200Error = _abi.MwaB200Error
-ALGO_AUTO, ALGO_SIMT, ALGO_TCGEN05, ALGO_TCGEN05_V1 = (_abi.ALGO_AUTO, _abi.ALGO_SIMT, _abi.ALGO_TCGEN05,
-                                                          _abi.ALGO_TCGEN05_V1)
+ALGO_AUTO, ALGO_SIMT, ALGO_TCGEN05 = _abi.ALGO_AUTO, _abi.ALGO_SIMT, _abi.ALGO_TCGEN05

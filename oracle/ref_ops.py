@@ -91,59 +91,32 @@ def window_keep(alpha: torch.Tensor, ws: int, s: int) -> torch.Tensor:
 # a2: window attention core   (layers/masked_win_attention.py:96-131)
 # --------------------------------------------------------------------------------------
 def window_attention(xw, qkv_w, qkv_b, proj_w, proj_b, bias_table, heads: int, ws: int,
-                     mask=None, qk_scale=None, operand_dtype=None):
-    """xw (K,N,C) -> (K,N,C).  mask: None or (K,N,N) additive (already per kept window).
-
-    operand_dtype=None restates the reference (fp32 everywhere).  operand_dtype=torch.float16 additionally
-    models where the tcgen05 kernel rounds its tensor-core OPERANDS (accumulation, bias, softmax stay in the
-    working precision): x, Wqkv (q rows pre-multiplied by the scale), q/k/v, the un-normalised probabilities,
-    the normalised head outputs and Wproj.  It is the yardstick for "the kernel computes what it was designed to
-    compute"; the distance between the two oracles is the documented precision cost of fp16 operands.
-    """
+                     mask=None, qk_scale=None):
+    """xw (K,N,C) -> (K,N,C).  mask: None or (K,N,N) additive (already per kept window)."""
     K, N, C = xw.shape
     d = C // heads
     scale = qk_scale or d ** -0.5
-    if operand_dtype is None:
-        rnd = lambda t: t
-    else:
-        rnd = lambda t: t.to(operand_dtype).to(t.dtype)
-    if operand_dtype is None:
-        qkv = xw @ qkv_w.t()
-        if qkv_b is not None:
-            qkv = qkv + qkv_b
-        qkv = qkv.reshape(K, N, 3, heads, d)
-        q = qkv[:, :, 0].permute(0, 2, 1, 3) * scale      # (K,h,N,d); the reference scales q after the projection
-    else:
-        w = qkv_w.clone()
-        w[:C] = w[:C] * scale                              # the kernel folds the scale into Wq / bq at prepare time
-        qkv = rnd(xw) @ rnd(w).t()
-        if qkv_b is not None:
-            b = qkv_b.clone()
-            b[:C] = b[:C] * scale
-            qkv = qkv + b
-        qkv = rnd(qkv).reshape(K, N, 3, heads, d)
-        q = qkv[:, :, 0].permute(0, 2, 1, 3)
+    qkv = xw @ qkv_w.t()
+    if qkv_b is not None:
+        qkv = qkv + qkv_b
+    qkv = qkv.reshape(K, N, 3, heads, d)
+    q = qkv[:, :, 0].permute(0, 2, 1, 3) * scale      # (K,h,N,d); the reference scales q after the projection
     k = qkv[:, :, 1].permute(0, 2, 1, 3)
     v = qkv[:, :, 2].permute(0, 2, 1, 3)
     s_ = torch.einsum("khid,khjd->khij", q, k)
     s_ = s_ + expand_bias(bias_table, ws).to(s_.dtype)[None]
     if mask is not None:
         s_ = s_ + mask[:, None]
-    if operand_dtype is None:
-        p = torch.softmax(s_, dim=-1)
-        o = torch.einsum("khij,khjd->kihd", p, v).reshape(K, N, C)
-    else:
-        e = torch.exp(s_ - s_.amax(dim=-1, keepdim=True))
-        o = torch.einsum("khij,khjd->kihd", rnd(e), v) / e.sum(dim=-1).permute(0, 2, 1)[..., None]
-        o = rnd(o.reshape(K, N, C))
-    return o @ rnd(proj_w).t() + proj_b
+    p = torch.softmax(s_, dim=-1)
+    o = torch.einsum("khij,khjd->kihd", p, v).reshape(K, N, C)
+    return o @ proj_w.t() + proj_b
 
 
 # --------------------------------------------------------------------------------------
 # a1 / a6: the full block   (layers/masked_win_attention.py:169-251, win_attention.py:153-207)
 # --------------------------------------------------------------------------------------
 def masked_window_attention(x, alpha, qkv_w, qkv_b, proj_w, proj_b, bias_table,
-                            heads: int, ws: int, shift: int, qk_scale=None, operand_dtype=None):
+                            heads: int, ws: int, shift: int, qk_scale=None):
     """x (B,C,H,W), alpha (B,1,H,W) or None (= unmasked twin, every window kept) -> (B,C,H,W)."""
     assert 0 <= shift < ws, "shift_size must in 0-window_size"
     B, C, H, W = x.shape
@@ -162,7 +135,7 @@ def masked_window_attention(x, alpha, qkv_w, qkv_b, proj_w, proj_b, bias_table,
     y = torch.zeros_like(xw)
     if bool(keep.any()):
         y[keep] = window_attention(xw[keep], qkv_w, qkv_b, proj_w, proj_b, bias_table,
-                                   heads, ws, mask=mask, qk_scale=qk_scale, operand_dtype=operand_dtype)
+                                   heads, ws, mask=mask, qk_scale=qk_scale)
     ys = from_windows(y.reshape(-1, ws, ws, C), ws, H, W)
     if shift > 0:
         ys = torch.roll(ys, shifts=(shift, shift), dims=(1, 2))

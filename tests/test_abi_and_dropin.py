@@ -53,6 +53,8 @@ def test_argument_validation_without_gpu(lib):
     assert lib.mwa_forward(None, None, None, None, 1, 192, 8, 8, 8, 8, 0, 0, 0, None, None, 0, None) == -1
     assert lib.mwa_forward(one, None, one, one, 1, 192, 8, 8, 8, 8, 8, 0, 0, None, None, 0, None) == -1     # shift >= ws
     assert lib.mwa_forward(one, None, one, one, 1, 192, 12, 8, 8, 8, 0, 0, 0, None, None, 0, None) == -1    # H % ws
+    for algo in (3, 4, 5):                                                                          # unknown algo
+        assert lib.mwa_forward(None, None, None, None, 0, 192, 8, 8, 8, 8, 0, 0, algo, None, None, 0, None) == -1
     assert lib.mwa_workspace_bytes(16, 128, 192, 8) >= 5 * 6144
     assert lib.gdn_forward(None, None, None, 1, 192, 64, 0, 0, 0, None) == -1
     assert lib.gdn_forward(one, one, one, 0, 192, 64, 0, 0, 0, None) == 0                          # empty batch

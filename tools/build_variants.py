@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Development tool: side-by-side variants of one kernel source for A/B timing in a single GPU call.
 
-    python tools/build_variants.py mwa_ws.cu name1:-DKNOB=1,-DOTHER=2 name2:-DKNOB=3 ...
+    python tools/build_variants.py mwa_sp.cu notma:-DMWA_SP_NO_TMA=1 nostore:-DMWA_SP_EPI_NOSTORE=1 ...
 
 Each variant recompiles the named source with its defines, links it with the objects of the regular build and writes
 build/variants/<name>.so (git-ignored; travels to the GPU box).  `tools/kbench.py --lib build/variants/<name>.so` times it.

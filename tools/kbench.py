@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Kernel micro-benchmarks (development tool, run on the B200 box):
 times each hot-path kernel alone with CUDA events at the BASELINE config-2 shapes, prints the roofline
-fraction, and cross-checks the tcgen05 kernels against the fp32 SIMT kernels on the same inputs.
+fraction, and cross-checks the default kernels against the fp32 SIMT kernels on the same inputs.
 
     python tools/kbench.py [gdn] [attn] [round] [--iters 20]
 """
@@ -102,7 +102,7 @@ def bench_attn(args, dev, flush):
             flops = kept * R.flops_per_window(C, ws)
             byts = nwin * (2 * ws * ws * C * 4 + ws * ws * 4)
             res = {}
-            algos = [("tc-v1", pkg.ALGO_TCGEN05_V1), ("tcgen05", pkg.ALGO_TCGEN05)]
+            algos = [("auto", pkg.ALGO_AUTO)]
             if not args.no_simt:
                 algos.insert(0, ("simt", pkg.ALGO_SIMT))
             for name, algo in algos:
@@ -125,14 +125,13 @@ def bench_attn(args, dev, flush):
                 with torch.no_grad():
                     yu = mu(x)
                     med, best = timeit(lambda: mu(x), args.iters, flush)
-                print(f"attn C={C} h={heads} ws={ws} s={s} unmasked twin       tcgen05  median {med:8.3f} ms best {best:8.3f} "
+                print(f"attn C={C} h={heads} ws={ws} s={s} unmasked twin       auto     median {med:8.3f} ms best {best:8.3f} "
                       f"{flops / med / 1e9:8.1f} TFLOP/s = {flops / med / 1e9 / PEAKS['bf16_tflops'] * 100:5.2f}% tensor peak; "
-                      f"max |unmasked - masked(alpha=1)| {(yu - res['tcgen05']).abs().max().item():.1e}", flush=True)
-            base = "simt" if "simt" in res else "tc-v1"
-            if base in res and "tcgen05" in res:
-                d = (res[base] - res["tcgen05"]).abs()
-                print(f"    tcgen05 vs {base}: max abs diff {d.max().item():.3e}, "
-                      f"allclose(1e-3,1e-4) {torch.allclose(res['tcgen05'], res[base], rtol=1e-3, atol=1e-4)}",
+                      f"max |unmasked - masked(alpha=1)| {(yu - res['auto']).abs().max().item():.1e}", flush=True)
+            if "simt" in res and "auto" in res:
+                d = (res["simt"] - res["auto"]).abs()
+                print(f"    auto vs simt: max abs diff {d.max().item():.3e}, "
+                      f"allclose(1e-3,1e-4) {torch.allclose(res['auto'], res['simt'], rtol=1e-3, atol=1e-4)}",
                       flush=True)
 
 
