@@ -82,6 +82,11 @@ _SIGNATURES = {
                                            c_int64]),
     "rans_decode_with_indexes": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_int, c_void_p, c_void_p,
                                          c_int, c_void_p]),
+    "rans_lanes_encode": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int, c_void_p, c_int, c_void_p, c_void_p, c_int,
+                                  c_void_p, c_int64, c_void_p, c_void_p]),
+    "rans_lanes_pack": (c_int, [c_void_p, c_int64, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
+    "rans_lanes_decode": (c_int, [c_void_p, c_int64, c_void_p, c_int, c_void_p, c_int, c_void_p, c_int64, c_int64, c_void_p,
+                                  c_int, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
     "rate_workspace_bytes": (c_int64, [c_int]),
     "rate_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int64,
                              c_void_p, c_void_p, c_int, c_int64, c_void_p, c_int64, c_void_p, c_void_p]),

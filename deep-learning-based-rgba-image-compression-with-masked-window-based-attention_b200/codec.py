@@ -197,26 +197,49 @@ class EntropyBottleneck(nn.Module):
     def _symbols(self, z):
         return torch.round(z - self._get_medians()).to(torch.int32)
 
+    def _indexes(self, B, H, W, device=None):
+        """the table index of every element: its channel"""
+        C = self.channels
+        return torch.arange(C, dtype=torch.int32, device=device).view(1, C, 1).expand(B, C, H * W).reshape(B, -1)
+
     @torch.no_grad()
-    def compress(self, z):
-        """one string per image: the channel is the table index (models/AutoEncoderRGB_Journal.py:319)"""
+    def compress(self, z, coder="host", lanes=None):
+        """one string per image: the channel is the table index (models/AutoEncoderRGB_Journal.py:319).  coder="host": the
+        host rANS coder; "device": the lane-interleaved format coded on the GPU (`lanes` lanes, entropy.default_lanes if
+        None)"""
         if getattr(self, "_table", None) is None:
             self.update()
         B, C, H, W = z.shape
+        if coder == "device":
+            return self._table.encode_lanes(self._symbols(z).reshape(B, -1), self._indexes(B, H, W, z.device), lanes).strings()
+        if coder != "host":
+            raise ValueError(f"coder must be 'host' or 'device' (got {coder!r})")
         sym = self._symbols(z).cpu().numpy()
-        idx = torch.arange(C, dtype=torch.int32).view(C, 1, 1).expand(C, H, W).contiguous().numpy()
+        idx = self._indexes(1, H, W)[0].numpy()
         return [self._table.encode(sym[b], idx) for b in range(B)]
 
     @torch.no_grad()
     def decompress(self, strings, size):
-        """(:320, :372): symbols + medians"""
+        """(:320, :372): symbols + medians; the format of the strings picks the decoder"""
+        from . import entropy
         if getattr(self, "_table", None) is None:
             self.update()
+        if entropy.stream_format(strings) == "device":
+            streams = entropy.LaneStreams([strings], self.quantiles.device)
+            z_hat = self._decode_lanes(streams.decoder(self._table, 0), size)
+            streams.check()
+            return z_hat
         C, (H, W) = self.channels, size
-        idx = torch.arange(C, dtype=torch.int32).view(C, 1, 1).expand(C, H, W).contiguous().numpy()
+        idx = self._indexes(1, H, W)[0].numpy()
         sym = [torch.from_numpy(self._table.decoder(st).decode(idx)).view(1, C, H, W) for st in strings]
         dev = self.quantiles.device
         return torch.cat(sym, 0).to(dev).float() + self._get_medians()
+
+    def _decode_lanes(self, decoder, size):
+        """z_hat from a LaneDecoder over its strings, on the GPU; its LaneStreams.check() is the caller's"""
+        B, (H, W) = decoder.count, size
+        sym = decoder.decode(self._indexes(B, H, W, self.quantiles.device).contiguous())
+        return sym.view(B, self.channels, H, W).float() + self._get_medians()
 
     def likelihood(self, z_hat):
         B, C = z_hat.shape[:2]
@@ -233,6 +256,7 @@ class GaussianConditional(nn.Module):
     def __init__(self, scale_table=None):
         super().__init__()
         self.scale_table, self._table = None, None
+        self._scale_table_copies = {}
 
     def update_scale_table(self, scale_table, force=False):
         """one quantised Gaussian CDF per scale level (CompressAI's GaussianConditional.update_scale_table + update)"""
@@ -240,12 +264,16 @@ class GaussianConditional(nn.Module):
         if self._table is not None and not force:
             return False
         self.scale_table = torch.as_tensor(scale_table, dtype=torch.float32).clone()
+        self._scale_table_copies = {}
         self._table = entropy.gaussian_table(self.scale_table)
         return True
 
     def build_indexes(self, scales):
+        """the scale table is copied to the scales' device once (a copy per call would synchronise every slice)"""
         from . import entropy
-        return entropy.build_indexes(scales, self.scale_table)
+        if scales.device not in self._scale_table_copies:
+            self._scale_table_copies[scales.device] = self.scale_table.to(scales.device)
+        return entropy.build_indexes(scales, self._scale_table_copies[scales.device])
 
     @staticmethod
     def likelihood(y, scales, means):
@@ -404,37 +432,63 @@ class AutoEncoder(nn.Module):
         return updated
 
     @torch.no_grad()
-    def compress(self, input, mask):
+    def compress(self, input, mask, coder="host", lanes=None):
         """models/AutoEncoderRGB_Journal.py:312-368.  The device side is the forward's own pieces (analysis, hyperprior,
-        fused slice loop: one pass gives every slice's mu, scale and y_hat); symbols and table indexes of all slices go to
-        the host in ONE copy and the rANS coder runs there (csrc/rans.cu), one string per image (for a batch of one this is
-        the reference's structure; the reference puts a whole batch into one string and can only decompress batch 1)."""
+        fused slice loop: one pass gives every slice's mu, scale and y_hat); one string per image (for a batch of one this
+        is the reference's structure; the reference puts a whole batch into one string and can only decompress batch 1).
+        coder="host": symbols and table indexes of all slices go to the host in ONE copy and the rANS coder runs there
+        (csrc/rans.cu).  coder="device": the lane-interleaved format (DESIGN.md 4.7), coded on the GPU with `lanes` lanes
+        per string (entropy.default_lanes of the message if None); only the finished strings cross to the host."""
+        if coder not in ("host", "device"):
+            raise ValueError(f"coder must be 'host' or 'device' (got {coder!r})")
         self.update()
         _, me = alpha_pyramid(mask, 3)
         y = self.Encoder(input, mask, None, me[1], me[2], None)
         z = self.h_a(y)
-        z_strings = self.entropy_bottleneck.compress(z)
-        z_hat = self.entropy_bottleneck.decompress(z_strings, z.shape[-2:])
+        eb = self.entropy_bottleneck
+        if coder == "device":
+            # z_hat is what the decoder will reconstruct from the z strings: their symbols + the medians
+            B, _, Hz, Wz = z.shape
+            z_sym = eb._symbols(z)
+            z_job = eb._table.encode_lanes(z_sym.reshape(B, -1), eb._indexes(B, Hz, Wz, z.device), lanes)
+            z_hat = z_sym.float() + eb._get_medians()
+        else:
+            z_strings = eb.compress(z)
+            z_hat = eb.decompress(z_strings, z.shape[-2:])
         latent_scales, latent_means = self.h_scale_s(z_hat), self.h_mean_s(z_hat)
         _, means, scales = self.slice_loop(y, latent_means, latent_scales)
-        symbols = torch.round(y - means).to(torch.int32).cpu().numpy()          # quantize(y, "symbols", mu)   (:347)
-        indexes = self.gaussian_conditional.build_indexes(scales).cpu().numpy()
+        symbols = torch.round(y - means).to(torch.int32)                       # quantize(y, "symbols", mu)   (:347)
+        indexes = self.gaussian_conditional.build_indexes(scales)
         table = self.gaussian_conditional._table
+        if coder == "device":
+            B = y.shape[0]
+            y_job = table.encode_lanes(symbols.reshape(B, -1), indexes.reshape(B, -1), lanes)
+            return {"strings": [y_job.strings(), z_job.strings()], "shape": z.shape[-2:]}
+        symbols, indexes = symbols.cpu().numpy(), indexes.cpu().numpy()
         y_strings = [table.encode(symbols[b], indexes[b]) for b in range(y.shape[0])]
         return {"strings": [y_strings, z_strings], "shape": z.shape[-2:]}
 
     @torch.no_grad()
     def decompress(self, strings, shape, mask):
         """models/AutoEncoderRGB_Journal.py:370-415: slice by slice -- mu and scale of slice i need the decoded slices < i --
-        with the same kernels as the encoder, so the tables' indexes and the reconstruction are bit-identical to its."""
+        with the same kernels as the encoder, so the tables' indexes and the reconstruction are bit-identical to its.
+        The strings' format picks the decoder: host-format strings are decoded on the host, slice by slice; lane-format
+        strings are staged on the GPU in one copy and decoded there, with one synchronisation (the status check) in all."""
+        from . import entropy
         from .layers.conv import split_into
         self.update()
-        z_hat = self.entropy_bottleneck.decompress(strings[1], shape)
+        eb, table = self.entropy_bottleneck, self.gaussian_conditional._table
+        streams = None
+        if entropy.stream_format(list(strings[0]) + list(strings[1])) == "device":
+            streams = entropy.LaneStreams([strings[1], strings[0]], eb.quantiles.device)
+            z_hat = eb._decode_lanes(streams.decoder(eb._table, 0), shape)
+            y_decoder = streams.decoder(table, 1)
+        else:
+            z_hat = eb.decompress(strings[1], shape)
+            decoders = [table.decoder(st) for st in strings[0]]
         latent_scales, latent_means = self.h_scale_s(z_hat), self.h_mean_s(z_hat)
         B, M, H, W = latent_means.shape
         sl, ms, dev = M // self.num_slices, self.max_support_slices, latent_means.device
-        table = self.gaussian_conditional._table
-        decoders = [table.decoder(st) for st in strings[0]]
         fused = self.cc_mean_transforms[0][0].input_ps(latent_means) is not None
         if fused:
             mean_sup = split_into(latent_means, SplitAct.empty(B, M, H, W, 1, dev, channels=M + (ms + 1) * sl))
@@ -450,8 +504,12 @@ class AutoEncoder(nn.Module):
                 support = y_hat_slices[:ms]
                 mu = self.cc_mean_transforms[i](torch.cat([latent_means] + support, 1))
                 scale = self.cc_scale_transforms[i](torch.cat([latent_scales] + support, 1))
-            idx = self.gaussian_conditional.build_indexes(scale).cpu().numpy()
-            sym = torch.from_numpy(np.stack([decoders[b].decode(idx[b]) for b in range(B)])).view(B, sl, H, W)
+            idx = self.gaussian_conditional.build_indexes(scale)
+            if streams is not None:
+                sym = y_decoder.decode(idx.reshape(B, -1)).view(B, sl, H, W)
+            else:
+                idx = idx.cpu().numpy()
+                sym = torch.from_numpy(np.stack([decoders[b].decode(idx[b]) for b in range(B)])).view(B, sl, H, W)
             y_hat = sym.to(dev).float() + mu                                   # dequantize(rv, mu)   (:395)
             if fused:
                 split_into(y_hat, mean_sup, slot)
@@ -465,6 +523,8 @@ class AutoEncoder(nn.Module):
             y_hat_slices.append(y_hat)
         _, md = alpha_pyramid(mask, 3)
         x_hat = self.Decoder(torch.cat(y_hat_slices, 1), mask, None, md[1], md[2], None).clamp_(0, 1)
+        if streams is not None:
+            streams.check()
         return {"x_hat": x_hat}
 
     def detail(self, input, mask, reconmask, me2=None, me3=None):

@@ -8,76 +8,26 @@
 //   raw = -2 v - 1 (v < 0)   |   2 (v - max) (v >= max).
 // Symbols are pushed in order and coded in reverse so that the decoder reads them forward.  Parity with CompressAI's own
 // byte stream is UNPINNED (nothing to compare against); what is tested is the round trip and the stream length against
-// the entropy model's estimate.  The coder is serial by construction (one state per stream) and runs on the host.
+// the entropy model's estimate.  The coder is serial by construction (one state per stream) and runs on the host; its core
+// (rans.cuh) is shared with the device coder of the lane-interleaved format (rans_dev.cu), whose lanes are streams of
+// exactly this kind.
 #include <cstdint>
 #include <cstring>
 #include <vector>
+#include "rans.cuh"
 #include "status.cuh"
 
-namespace b200 {
-namespace {
-
-constexpr int kPrecision = 16, kBypassPrecision = 4, kMaxBypass = (1 << kBypassPrecision) - 1;
-constexpr uint64_t kRansL = uint64_t(1) << 31;          // lower bound of the normalisation interval
-
-struct Sym {
-    uint16_t start, range;
-    bool bypass;
-};
-
-inline void enc_put(uint64_t& x, std::vector<uint32_t>& out, uint32_t start, uint32_t freq, uint32_t scale_bits) {
-    const uint64_t x_max = ((kRansL >> scale_bits) << 32) * freq;
-    if (x >= x_max) {
-        out.push_back(uint32_t(x));
-        x >>= 32;
-    }
-    x = ((x / freq) << scale_bits) + (x % freq) + start;
-}
-inline void enc_put_bits(uint64_t& x, std::vector<uint32_t>& out, uint32_t val, uint32_t nbits) {
-    const uint64_t x_max = (kRansL >> nbits) << 32;
-    if (x >= x_max) {
-        out.push_back(uint32_t(x));
-        x >>= 32;
-    }
-    x = (x << nbits) | val;
-}
-
-struct Decoder {
-    const uint32_t* p;
-    const uint32_t* end;
-    uint64_t x;
-    bool ok;
-    void init(const uint32_t* s, int64_t nwords) {
-        p = s; end = s + nwords; ok = nwords >= 2;
-        x = 0;
-        if (ok) {
-            x = uint64_t(p[0]) | (uint64_t(p[1]) << 32);
-            p += 2;
-        }
-    }
-    inline void renorm() {
-        if (x < kRansL) {
-            if (p < end) x = (x << 32) | *p++;
-            else ok = false;
-        }
-    }
-    inline uint32_t get(uint32_t bits) const { return uint32_t(x & ((uint64_t(1) << bits) - 1)); }
-    inline void advance(uint32_t start, uint32_t freq, uint32_t bits) {
-        x = freq * (x >> bits) + (x & ((uint64_t(1) << bits) - 1)) - start;
-        renorm();
-    }
-    inline uint32_t get_bits(uint32_t nbits) {
-        const uint32_t v = uint32_t(x & ((uint64_t(1) << nbits) - 1));
-        x >>= nbits;
-        renorm();
-        return v;
-    }
-};
-
-}  // namespace
-}  // namespace b200
-
 using namespace b200;
+
+namespace {
+struct VectorEmit {
+    std::vector<uint32_t>& words;
+    bool operator()(uint32_t w) {
+        words.push_back(w);
+        return true;
+    }
+};
+}  // namespace
 
 extern "C" {
 
@@ -86,46 +36,17 @@ extern "C" {
 MWA_API int64_t rans_encode_with_indexes(const int32_t* symbols, const int32_t* indexes, int64_t n, const int32_t* cdfs, int cdf_stride,
                                  const int32_t* cdf_sizes, const int32_t* offsets, int ncdf, uint8_t* out, int64_t out_capacity) {
     if (n < 0 || (n > 0 && (!symbols || !indexes)) || !cdfs || !cdf_sizes || !offsets || !out || ncdf <= 0) return MWA_ERR_INVALID;
-    std::vector<Sym> syms;
-    syms.reserve(size_t(n) + 16);
-    for (int64_t i = 0; i < n; ++i) {
-        const int idx = indexes[i];
-        if (idx < 0 || idx >= ncdf) return MWA_ERR_INVALID;
-        const int32_t* cdf = cdfs + int64_t(idx) * cdf_stride;
-        const int32_t max_value = cdf_sizes[idx] - 2;
-        if (max_value < 0 || cdf_sizes[idx] > cdf_stride) return MWA_ERR_INVALID;
-        int32_t value = symbols[i] - offsets[idx];
-        uint32_t raw = 0;
-        if (value < 0) {
-            raw = uint32_t(-2 * int64_t(value) - 1);
-            value = max_value;
-        } else if (value >= max_value) {
-            raw = uint32_t(2 * (int64_t(value) - max_value));
-            value = max_value;
-        }
-        const int32_t lo = cdf[value], hi = cdf[value + 1];
-        if (hi <= lo) return MWA_ERR_INVALID;                   // zero-probability symbol: the table is broken
-        syms.push_back({uint16_t(lo), uint16_t(hi - lo), false});
-        if (value == max_value) {
-            int32_t ndig = 0;
-            while ((raw >> (ndig * kBypassPrecision)) != 0) ++ndig;
-            int32_t v = ndig;
-            while (v >= kMaxBypass) {
-                syms.push_back({uint16_t(kMaxBypass), 1, true});
-                v -= kMaxBypass;
-            }
-            syms.push_back({uint16_t(v), 1, true});
-            for (int32_t j = 0; j < ndig; ++j)
-                syms.push_back({uint16_t((raw >> (j * kBypassPrecision)) & kMaxBypass), 1, true});
-        }
-    }
+    // validate and code in one backward pass (the coder runs in reverse; an error discards the partial result)
     std::vector<uint32_t> words;
-    words.reserve(syms.size() / 2 + 4);
-    uint64_t x = kRansL;
-    for (size_t k = syms.size(); k-- > 0;) {
-        const Sym& s = syms[k];
-        if (s.bypass) enc_put_bits(x, words, s.start, kBypassPrecision);
-        else enc_put(x, words, s.start, s.range, kPrecision);
+    words.reserve(size_t(n) / 2 + 4);
+    VectorEmit emit{words};
+    uint64_t x = rans::kRansL;
+    for (int64_t i = n; i-- > 0;) {
+        const int idx = indexes[i];
+        if (idx < 0 || idx >= ncdf || cdf_sizes[idx] > cdf_stride) return MWA_ERR_INVALID;
+        if (rans::encode_element_reversed(x, emit, symbols[i], cdfs + int64_t(idx) * cdf_stride, cdf_sizes[idx],
+                                          offsets[idx]) != rans::kOk)
+            return MWA_ERR_INVALID;
     }
     words.push_back(uint32_t(x >> 32));
     words.push_back(uint32_t(x));
@@ -148,12 +69,13 @@ MWA_API int rans_decode_with_indexes(const uint8_t* stream, int64_t nbytes, int6
     if (!stream || !state || n < 0 || (n > 0 && (!indexes || !symbols_out)) || !cdfs || !cdf_sizes || !offsets || nbytes % 4 != 0)
         return MWA_ERR_INVALID;
     const uint32_t* w = reinterpret_cast<const uint32_t*>(stream);
-    Decoder d;
+    rans::Decoder d;
     if (state[0] == 0) {
-        d.init(w, nbytes / 4);            // first two words = the final encoder state (low half, high half)
+        d.init(w, 0, nbytes / 4);
     } else {
-        d.p = w + state[1];
-        d.end = w + nbytes / 4;
+        d.w = w;
+        d.p = state[1];
+        d.end = nbytes / 4;
         d.x = uint64_t(state[2]);
         d.ok = true;
     }
@@ -161,37 +83,11 @@ MWA_API int rans_decode_with_indexes(const uint8_t* stream, int64_t nbytes, int6
     for (int64_t i = 0; i < n; ++i) {
         const int idx = indexes[i];
         if (idx < 0 || idx >= ncdf) return MWA_ERR_INVALID;
-        const int32_t* cdf = cdfs + int64_t(idx) * cdf_stride;
-        const int32_t size = cdf_sizes[idx], max_value = size - 2;
-        const uint32_t cum = d.get(kPrecision);
-        // last entry <= cum (entries are increasing; the table is short: binary search)
-        int lo = 0, hi = size - 1;
-        while (hi - lo > 1) {
-            const int mid = (lo + hi) >> 1;
-            if (uint32_t(cdf[mid]) <= cum) lo = mid;
-            else hi = mid;
-        }
-        const int32_t s = lo;
-        d.advance(uint32_t(cdf[s]), uint32_t(cdf[s + 1] - cdf[s]), kPrecision);
-        int32_t value = s;
-        if (value == max_value) {
-            int32_t v = int32_t(d.get_bits(kBypassPrecision));
-            int32_t ndig = v;
-            while (v == kMaxBypass) {
-                v = int32_t(d.get_bits(kBypassPrecision));
-                ndig += v;
-            }
-            uint32_t raw = 0;
-            for (int32_t j = 0; j < ndig; ++j) raw |= d.get_bits(kBypassPrecision) << (j * kBypassPrecision);
-            value = int32_t(raw >> 1);
-            if (raw & 1) value = -value - 1;
-            else value += max_value;
-        }
-        if (!d.ok) return MWA_ERR_INVALID;
-        symbols_out[i] = value + offsets[idx];
+        if (!rans::decode_element(d, cdfs + int64_t(idx) * cdf_stride, cdf_sizes[idx], offsets[idx], symbols_out[i]))
+            return MWA_ERR_INVALID;
     }
     state[0] = 1;
-    state[1] = int64_t(d.p - w);
+    state[1] = d.p;
     state[2] = int64_t(d.x);
     return MWA_OK;
 }

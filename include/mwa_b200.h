@@ -337,6 +337,41 @@ MWA_API int rans_decode_with_indexes(const uint8_t* stream, int64_t nbytes, int6
                                      int ncdf, int32_t* symbols_out);
 
 /* ------------------------------------------------------------------------------------------------
+ * Lane-interleaved rANS on the device (csrc/rans_dev.cu; DESIGN.md 4.7)   the same coder as above, on the GPU, for a stream
+ *   format whose message is split across L lanes: element g of a stream (counted across all decode calls) belongs to lane
+ *   g mod L, and lane l's segment is byte for byte what rans_encode_with_indexes writes for elements l, l + L, l + 2L, ...
+ *   Stream layout, little-endian u32 words:
+ *     MWA_RANS_LANES_MAGIC, 0x80000000 | MWA_RANS_LANES_VERSION, L, L lane byte lengths (multiples of 4, >= 8), segments.
+ *   Word 1 has its top bit set; in a host-format stream word 1 is the high half of a final state in [2^31, 2^63), so < 2^31.
+ *   Device pointers, asynchronous on `stream`; tables as for the host coder (cdfs / cdf_sizes / offsets, device copies).
+ * rans_lanes_encode : symbols, indexes (n_streams, n) int32.  Thread (s, l) writes lane l of stream s into slot s * lanes + l
+ *             of `slots` (n_streams * lanes slots of slot_words u32 each; the segment ends at the slot's end) and sets
+ *             lane_words[s * lanes + l] to its length in words, or MWA_ERR_WORKSPACE when the slot is too small (nothing is
+ *             written past it: retry with larger slots), or MWA_ERR_INVALID for an index outside [0, ncdf) / a broken row.
+ * rans_lanes_pack   : after rans_lanes_encode on the same slots: writes every stream, header included, back to back into
+ *             `out` (out_words u32; n_streams * (3 + lanes + lanes * slot_words) always suffice), stream_bytes[s] = byte
+ *             length of stream s and stream_bytes[n_streams] = total bytes, or the negative status of a failed lane
+ *             (INVALID before WORKSPACE), in which case `out` holds no streams.  lane_dst: n_streams * lanes int64 scratch.
+ * rans_lanes_decode : data = the streams of the call (data_words u32); lane_state (total_lanes, 4) int64, one row per lane of
+ *             every stream: {x, next word, end word, stream + 2^32 lane}, prepared by the caller as {0, index of the lane
+ *             segment's first word in data, one past its last, ...} and updated by each call, so successive calls continue
+ *             each stream; stream_lanes[s] = L of stream s (streams may differ).  Decodes elements [position, position + n)
+ *             of every stream with indexes (n_streams, n) into symbols (n_streams, n).  A truncated or corrupt segment or
+ *             an index outside [0, ncdf) sets status[s] (int32, zeroed by the caller) to MWA_ERR_INVALID; that stream's
+ *             later lanes and calls stop, its symbols are then undefined.  The return value covers the arguments only. */
+#define MWA_RANS_LANES_MAGIC 0x4C41574Du   /* "MWAL" */
+#define MWA_RANS_LANES_VERSION 1u
+MWA_API int rans_lanes_encode(const int32_t* symbols, const int32_t* indexes, int n_streams, int64_t n, int lanes,
+                              const int32_t* cdfs, int cdf_stride, const int32_t* cdf_sizes, const int32_t* offsets,
+                              int ncdf, uint32_t* slots, int64_t slot_words, int32_t* lane_words, void* stream);
+MWA_API int rans_lanes_pack(const uint32_t* slots, int64_t slot_words, const int32_t* lane_words, int n_streams, int lanes,
+                            int64_t* lane_dst, int64_t* stream_bytes, uint32_t* out, int64_t out_words, void* stream);
+MWA_API int rans_lanes_decode(const uint32_t* data, int64_t data_words, int64_t* lane_state, int total_lanes,
+                              const int32_t* stream_lanes, int n_streams, const int32_t* indexes, int64_t n,
+                              int64_t position, const int32_t* cdfs, int cdf_stride, const int32_t* cdf_sizes,
+                              const int32_t* offsets, int ncdf, int32_t* symbols, int32_t* status, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Rate / distortion terms of the forward (csrc/rate.cu)   replaces  models/AutoEncoderRGB_Journal.py:36-64 (reconstruct_error)
  * and :283-291 (bits of y under the Gaussian conditional, of z under the factorised prior, bpp), which the reference runs
  * as ~90 elementwise / reduction / batched-GEMM launches: one pass per term + a finalize launch, inference only.
