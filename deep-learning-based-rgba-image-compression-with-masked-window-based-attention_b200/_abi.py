@@ -91,6 +91,8 @@ _SIGNATURES = {
     "rate_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int64,
                              c_void_p, c_void_p, c_int, c_int64, c_void_p, c_int64, c_void_p, c_void_p]),
     "mask_constraint_forward": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
+    "rgba8_ingest": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
+    "rgba8_egress": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 

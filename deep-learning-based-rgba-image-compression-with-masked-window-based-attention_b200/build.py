@@ -23,7 +23,7 @@ ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"]
 # per-file extra flags: the rounding kernels must round like torch's separate fp32 ops (no FMA contraction)
 EXTRA = {"round.cu": ["-fmad=false"], "alpha.cu": ["-fmad=false"], "rate.cu": ["-fmad=false"]}
-SOURCES = ["abi.cu", "round.cu", "gdn.cu", "gdn_tc.cu", "mwa.cu", "mwa_sp.cu", "mwa_small.cu", "mwa_bwd.cu", "gate.cu", "alpha.cu", "conv_tc.cu", "msssim.cu", "rans.cu", "rans_dev.cu", "rate.cu"]
+SOURCES = ["abi.cu", "round.cu", "gdn.cu", "gdn_tc.cu", "mwa.cu", "mwa_sp.cu", "mwa_small.cu", "mwa_bwd.cu", "gate.cu", "alpha.cu", "conv_tc.cu", "msssim.cu", "rans.cu", "rans_dev.cu", "rate.cu", "rgba8.cu"]
 
 
 def _nvcc() -> str:

@@ -24,6 +24,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from . import quant
+from . import rgba8 as rgba8_mod
 from .layers.GDN import GDN
 from .layers.Masked_Attention import Win_noShift_Attention, conv3x3
 from .layers.conv import ACT_ADD2, ACT_LRP, ACT_QUANT, ACT_RELU, Conv2d, ConvStack, ConvTranspose2d, SplitAct
@@ -474,6 +475,15 @@ class AutoEncoder(nn.Module):
         with the same kernels as the encoder, so the tables' indexes and the reconstruction are bit-identical to its.
         The strings' format picks the decoder: host-format strings are decoded on the host, slice by slice; lane-format
         strings are staged on the GPU in one copy and decoded there, with one synchronisation (the status check) in all."""
+        x_hat, streams = self._decode(strings, shape, mask)
+        x_hat = x_hat.clamp_(0, 1)
+        if streams is not None:
+            streams.check()
+        return {"x_hat": x_hat}
+
+    def _decode(self, strings, shape, mask):
+        """decompress up to the synthesis transform: (unclamped x_hat, the LaneStreams whose check() is the caller's, or
+        None for host-format strings)"""
         from . import entropy
         from .layers.conv import split_into
         self.update()
@@ -522,10 +532,41 @@ class AutoEncoder(nn.Module):
                 y_hat = quant.lrp_add(y_hat, self.lrp_transforms[i](torch.cat([latent_means] + y_hat_slices[:ms] + [y_hat], 1)))
             y_hat_slices.append(y_hat)
         _, md = alpha_pyramid(mask, 3)
-        x_hat = self.Decoder(torch.cat(y_hat_slices, 1), mask, None, md[1], md[2], None).clamp_(0, 1)
+        return self.Decoder(torch.cat(y_hat_slices, 1), mask, None, md[1], md[2], None), streams
+
+    @torch.no_grad()
+    def compress_rgba8(self, rgba8, coder="host", lanes=None):
+        """compress for 8-bit RGBA of any size: uint8 (B, H, W, 4) or (H, W, 4), on the GPU or the host (copied once).
+        The image is converted on the device to the planes the model was trained on (a / 255, colour premultiplied by the
+        binarised alpha; csrc/rgba8.cu) and padded at the bottom and right with transparent pixels to multiples of 64, then
+        compressed as `compress` does; the stream format is unchanged.  Returns {"strings", "shape", "size": (H, W)}."""
+        if coder not in ("host", "device"):
+            raise ValueError(f"coder must be 'host' or 'device' (got {coder!r})")
+        rgba8_mod.as_batch(rgba8, (4,), "rgba8")
+        image, alpha, size = rgba8_mod.rgba8_ingest(rgba8, self.entropy_bottleneck.quantiles.device)
+        out = self.compress(image, alpha, coder=coder, lanes=lanes)
+        out["size"] = size
+        return out
+
+    @torch.no_grad()
+    def decompress_rgba8(self, strings, shape, alpha8):
+        """decompress to uint8 (B, H, W, 4).  alpha8: uint8 (B, H, W) or (H, W), the images' alpha (the decoder takes it as
+        `decompress` takes the mask); it gives the original size, and shape must be (ceil(H / 64), ceil(W / 64)).  Alpha is
+        copied through; RGB = rint(clamp(x_hat, 0, 1) * 255) where alpha > 0, else 0, cropped to H x W in one launch."""
+        a8 = rgba8_mod.as_batch(alpha8.unsqueeze(-1) if isinstance(alpha8, torch.Tensor) else alpha8, (1,), "alpha8")
+        B, H, W, _ = a8.shape
+        want = (rgba8_mod.padded(H) // rgba8_mod.PAD, rgba8_mod.padded(W) // rgba8_mod.PAD)
+        if tuple(int(v) for v in shape) != want:
+            raise ValueError(f"shape {tuple(shape)} does not fit a {H} x {W} alpha: expected {want}")
+        if len(strings) != 2 or len(strings[0]) != B or len(strings[1]) != B:
+            raise ValueError(f"expected [y strings, z strings] of {B} images each")
+        a8 = rgba8_mod.on_device(a8, self.entropy_bottleneck.quantiles.device)
+        _, alpha, _ = rgba8_mod.rgba8_ingest(a8)
+        x_hat, streams = self._decode(strings, shape, alpha)
+        out = rgba8_mod.rgba8_egress(x_hat, a8.view(B, H, W))
         if streams is not None:
             streams.check()
-        return {"x_hat": x_hat}
+        return out
 
     def detail(self, input, mask, reconmask, me2=None, me3=None):
         """every tensor of the forward the parity tests look at"""

@@ -1,0 +1,98 @@
+"""8-bit RGBA images of any size in and out of the codec (csrc/rgba8.cu, DESIGN.md 4.8).
+
+    rgba8_ingest(rgba8)          uint8 (B, H, W, 4) or (H, W, 4) -> fp32 image (B, 3, Hp, Wp), alpha (B, 1, Hp, Wp), (H, W)
+                                 uint8 (..., 1) (alpha only)     -> None, alpha, (H, W)
+    rgba8_egress(x_hat, alpha8)  fp32 (B, 3, Hp, Wp) + uint8 (B, H, W) -> uint8 (B, H, W, 4) on x_hat's device
+
+Hp / Wp are H / W rounded up to a multiple of 64 (the model's coarsest stride: z is Hp / 64 x Wp / 64); the padding, at the
+bottom and right, is transparent.  The planes are what the model was trained on: a / 255 and the colour premultiplied by
+the binarised alpha.  One kernel launch each way.
+"""
+from __future__ import annotations
+
+import torch
+
+from . import _abi
+
+PAD = 64
+# B * Hp * Wp * 48 (the forward's largest activation, 192 channels at 1/2 scale) must stay below 2^31: the C entry points'
+# guard, checked here too so that the planes are not allocated for an input they will refuse
+MAX_ELEMENTS = 2 ** 31
+
+
+def padded(n: int) -> int:
+    return -(-n // PAD) * PAD
+
+
+def _check_size(B: int, H: int, W: int) -> None:
+    if H < 1 or W < 1:
+        raise ValueError(f"image height and width must be >= 1 (got {H} x {W})")
+    if B * padded(H) * padded(W) * 48 >= MAX_ELEMENTS:
+        raise _abi.MwaB200Error(f"{B} x {H} x {W} is too large: B * Hp * Wp * 48 must stay below 2^31")
+
+
+def on_device(t: torch.Tensor, device) -> torch.Tensor:
+    """t on the CUDA device (the current one if None): one copy for a CPU tensor, non-blocking when it is pinned"""
+    if t.is_cuda and device is None:
+        return t
+    device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+    if device.type != "cuda":
+        raise _abi.MwaB200Error(f"8-bit images are converted on a CUDA device (got {device}); there is no CPU fallback")
+    return t.to(device, non_blocking=t.is_pinned())
+
+
+def as_batch(t: torch.Tensor, channels: tuple, what: str) -> torch.Tensor:
+    """uint8 (B, H, W, C) or (H, W, C) with C in `channels`, contiguous, as (B, H, W, C)"""
+    if not isinstance(t, torch.Tensor):
+        raise ValueError(f"{what} must be a torch.Tensor (got {type(t).__name__})")
+    if t.dtype != torch.uint8:
+        raise _abi.MwaB200Error(f"{what} must be uint8 (got {t.dtype})")
+    if t.dim() not in (3, 4) or t.shape[-1] not in channels:
+        raise ValueError(f"{what} must be (B, H, W, C) or (H, W, C) with C in {channels} (got {tuple(t.shape)})")
+    if not t.is_contiguous():
+        raise ValueError(f"{what} must be contiguous (interleaved channels, rows back to back)")
+    return t if t.dim() == 4 else t.unsqueeze(0)
+
+
+def rgba8_ingest(rgba8: torch.Tensor, device=None):
+    """(image, alpha, (H, W)): the fp32 planes of uint8 RGBA (C = 4; image None for C = 1, an alpha plane alone), padded to
+    multiples of 64.  A CPU input is copied to `device` (default: the current CUDA device) once."""
+    t = as_batch(rgba8, (1, 4), "rgba8")
+    B, H, W, C = t.shape
+    _check_size(B, H, W)
+    t = on_device(t, device)
+    if t.data_ptr() % 4:
+        t = t.clone()
+    Hp, Wp = padded(H), padded(W)
+    alpha = torch.empty(B, 1, Hp, Wp, dtype=torch.float32, device=t.device)
+    image = torch.empty(B, 3, Hp, Wp, dtype=torch.float32, device=t.device) if C == 4 else None
+    lib = _abi.load()
+    with torch.cuda.device(t.device):
+        _abi.check(lib.rgba8_ingest(t.data_ptr(), _abi.ptr(image), alpha.data_ptr(), B, H, W, C, _abi.stream_handle()),
+                   "rgba8_ingest")
+    _abi.count_launches(1)
+    return image, alpha, (H, W)
+
+
+def rgba8_egress(x_hat: torch.Tensor, alpha8: torch.Tensor) -> torch.Tensor:
+    """uint8 (B, H, W, 4) from the decoder's fp32 (B, 3, Hp, Wp) x_hat (unclamped) and the uint8 (B, H, W) alpha: A = alpha,
+    RGB = rint(clamp(x_hat, 0, 1) * 255) where alpha > 0, else 0"""
+    _abi.require_cuda_f32(x_hat, "x_hat")
+    if alpha8.dtype != torch.uint8 or alpha8.dim() != 3 or not alpha8.is_contiguous():
+        raise ValueError(f"alpha8 must be contiguous uint8 (B, H, W) (got {alpha8.dtype} {tuple(alpha8.shape)})")
+    B, H, W = alpha8.shape
+    _check_size(B, H, W)
+    if tuple(x_hat.shape) != (B, 3, padded(H), padded(W)):
+        raise ValueError(f"x_hat must be (B, 3, Hp, Wp) = {(B, 3, padded(H), padded(W))} for alpha {tuple(alpha8.shape)} "
+                         f"(got {tuple(x_hat.shape)})")
+    alpha8 = on_device(alpha8, x_hat.device)
+    x_hat = x_hat.contiguous()
+    if x_hat.data_ptr() % 16:
+        x_hat = x_hat.clone()
+    out = torch.empty(B, H, W, 4, dtype=torch.uint8, device=x_hat.device)
+    lib = _abi.load()
+    with torch.cuda.device(x_hat.device):
+        _abi.check(lib.rgba8_egress(x_hat.data_ptr(), alpha8.data_ptr(), out.data_ptr(), B, H, W, _abi.stream_handle()),
+                   "rgba8_egress")
+    _abi.count_launches(1)
+    return out

@@ -385,6 +385,24 @@ MWA_API int rate_forward(const float* input, const float* x_hat, const float* ma
                  const float* scales, const float* means, int64_t n_y, const float* z_hat, const float* const* eb_params,
                  int Cz, int64_t hw_z, void* workspace, int64_t workspace_bytes, float* out4, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * 8-bit RGBA images of any size (csrc/rgba8.cu; DESIGN.md 4.8)   replaces the caller's conversion around compress /
+ *   decompress (my_datasets: ToTensor + premultiplication by the binarised alpha; after decoding: clamp, quantise, interleave)
+ *   and pads to the model's geometry, Hp = 64 * ceil(H / 64), Wp = 64 * ceil(W / 64) (z is Hp / 64 x Wp / 64).
+ * rgba8_ingest : rgba8 uint8 (B, H, W, C) contiguous, C = 4 (RGBA) or 1 (alpha only) -> alpha fp32 (B, 1, Hp, Wp) and, for
+ *                C = 4, image fp32 (B, 3, Hp, Wp) (image is not touched and may be NULL for C = 1).  For y < H, x < W:
+ *                  alpha = a / 255;   image_c = rgb_c / 255 if a > 0, else 0      (IEEE round-to-nearest divisions)
+ *                every other element (bottom and right padding) is +0.0: transparent.
+ * rgba8_egress : x_hat fp32 (B, 3, Hp, Wp), alpha8 uint8 (B, H, W) -> rgba8 uint8 (B, H, W, 4), per pixel:
+ *                  A = alpha8;   RGB = rint(clamp(x_hat, 0, 1) * 255) (fp32 multiply, half to even; NaN -> 0) if A > 0, else 0
+ * MWA_ERR_INVALID before any CUDA call: B < 0, H < 1, W < 1, C not in {1, 4}, or B * Hp * Wp * 48 >= 2^31 (the forward's
+ *   largest activation, 192 channels at 1/2 scale, must stay within int32 element indexing); then, for B > 0, a NULL
+ *   pointer.  MWA_ERR_ALIGNMENT: an fp32 plane not 16-byte aligned, or an RGBA buffer not 4-byte aligned.
+ *   B = 0 returns MWA_OK and launches nothing.  One launch each, no allocation, no synchronisation.
+ * ------------------------------------------------------------------------------------------------ */
+MWA_API int rgba8_ingest(const uint8_t* rgba8, float* image, float* alpha, int B, int H, int W, int C, void* stream);
+MWA_API int rgba8_egress(const float* x_hat, const uint8_t* alpha8, uint8_t* rgba8, int B, int H, int W, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -27,6 +27,7 @@ codec = importlib.import_module(PACKAGE_NAME + ".codec")
 metrics = importlib.import_module(PACKAGE_NAME + ".metrics")
 pipeline = importlib.import_module(PACKAGE_NAME + ".pipeline")
 _params = importlib.import_module(PACKAGE_NAME + ".layers._params")
+rgba8 = importlib.import_module(PACKAGE_NAME + ".rgba8")
 
 GDN = GDN_mod.GDN
 LowerBound = GDN_mod.LowerBound
@@ -53,5 +54,7 @@ masked_ms_ssim = metrics.masked_ms_ssim
 masked_psnr = metrics.masked_psnr
 HostPipeline = pipeline.HostPipeline
 invalidate_param_blocks = _params.invalidate_param_blocks
+rgba8_ingest = rgba8.rgba8_ingest
+rgba8_egress = rgba8.rgba8_egress
 MwaB200Error = _abi.MwaB200Error
 ALGO_AUTO, ALGO_SIMT, ALGO_TCGEN05 = _abi.ALGO_AUTO, _abi.ALGO_SIMT, _abi.ALGO_TCGEN05
