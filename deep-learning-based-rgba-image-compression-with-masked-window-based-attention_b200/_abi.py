@@ -78,6 +78,8 @@ _SIGNATURES = {
                                       c_void_p]),
     "ms_ssim_pool_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,
                                      c_void_p]),
+    "ms_ssim_level_backward": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_float, c_void_p, c_void_p,
+                                       c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "rans_encode_with_indexes": (c_int64, [c_void_p, c_void_p, c_int64, c_void_p, c_int, c_void_p, c_void_p, c_int, c_void_p,
                                            c_int64]),
     "rans_decode_with_indexes": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_int, c_void_p, c_void_p,

@@ -10,6 +10,10 @@
 //                   per CTA.  HBM traffic = the two planes + the mask, once.
 //   ms_ssim_pool  : (X * m, Y * m, m) -> 2x2 average pools of all three in one pass.
 // fp32 like the reference; the sums are accumulated in a different order, so values agree to ~1e-6, not bit for bit.
+//   ms_ssim_level_bwd : the adjoint of one level (and of the pool that fed the next one), one launch per level from the
+//                   coarsest to the finest; see ms_ssim_level_bwd_kernel.  It shares the Gaussian taps (gauss_taps) and
+//                   the counted-position rule (counted) with ms_ssim_level, so it weights exactly the positions `counts`
+//                   counted.
 #include "common.cuh"
 #include "status.cuh"
 
@@ -23,6 +27,37 @@ constexpr int kIH = kTH + kApron, kIW = kTW + kApron;
 struct Gauss {
     float w[kWin];
 };
+
+// metrics/masked_ms_ssim_torch.py:13-24 (_fspecial_gauss_1d) in fp32; symmetric bit for bit (w[i] == w[10 - i])
+Gauss gauss_taps() {
+    Gauss g;
+    float s = 0.f;
+    for (int i = 0; i < kWin; ++i) {
+        const float c = float(i - kWin / 2);
+        g.w[i] = expf(-(c * c) / (2.f * 1.5f * 1.5f));
+        s += g.w[i];
+    }
+    for (int i = 0; i < kWin; ++i) g.w[i] /= s;
+    return g;
+}
+
+// per-level constants: SSIM's C1, C2 and the nearest-resize ratios of the valid region
+struct Level {
+    float C1, C2, scale_h, scale_w;
+};
+
+Level level_consts(int H, int W, float data_range) {
+    const int oh = H - kApron, ow = W - kApron;
+    return {(0.01f * data_range) * (0.01f * data_range), (0.03f * data_range) * (0.03f * data_range),
+            float(double(H) / oh), float(double(W) / ow)};
+}
+
+// n_p: whether valid-region position (yy, xx) is averaged: the nearest-resized mask of the valid region (:104-108),
+// source index floor(dst * in / out)
+__device__ __forceinline__ bool counted(const float* mp, int yy, int xx, int H, int W, float scale_h, float scale_w) {
+    const int my = min(int(floorf(float(yy) * scale_h)), H - 1), mx = min(int(floorf(float(xx) * scale_w)), W - 1);
+    return mp[int64_t(my) * W + mx] > 0.f;
+}
 
 __global__ void __launch_bounds__(256)
 ms_ssim_level_kernel(const float* __restrict__ X, const float* __restrict__ Y, const float* __restrict__ mask, int C, int H,
@@ -81,9 +116,7 @@ ms_ssim_level_kernel(const float* __restrict__ X, const float* __restrict__ Y, c
             const float s1 = m[2] - mu1 * mu1, s2 = m[3] - mu2 * mu2, s12 = m[4] - mu1 * mu2;
             const float cs = (2.f * s12 + C2) / (s1 + s2 + C2);
             const float ss = ((2.f * mu1 * mu2 + C1) / (mu1 * mu1 + mu2 * mu2 + C1)) * cs;
-            // nearest-resized mask of the valid region (:104-108): source index floor(dst * in / out)
-            const int my = min(int(floorf(float(yy) * scale_h)), H - 1), mx = min(int(floorf(float(xx) * scale_w)), W - 1);
-            if (mp[int64_t(my) * W + mx] > 0.f) {
+            if (counted(mp, yy, xx, H, W, scale_h, scale_w)) {
                 s_ssim += ss;
                 s_cs += cs;
                 s_n += 1.f;
@@ -150,6 +183,160 @@ ms_ssim_pool_kernel(const float* __restrict__ X, const float* __restrict__ Y, co
     }
 }
 
+// Backward of one level.  With Xm = X b, Ym = Y b (b = mask > 0), the valid blur G and, per valid position p, the maps of
+// the forward (mu1, mu2, s1, s2, s12, B1 = mu1^2 + mu2^2 + C1, B2 = s1 + s2 + C2, l = (2 mu1 mu2 + C1) / B1,
+// cs = (2 s12 + C2) / B2), the weight w_p = n_p / N_b of S[b,c] = sum_p w_p l_p cs_p and CS[b,c] = sum_p w_p cs_p gives
+//   g_cs = dS w l + dCS w,  g_l = dS w cs,  gE11 = gE22 = -g_cs cs / B2,  gE12 = 2 g_cs / B2,
+//   gmu1 = 2 g_l (mu2 - l mu1) / B1 - 2 mu1 gE11 - mu2 gE12     (gmu2: 1 <-> 2)
+//   dX = b (G^T gmu1 + 2 Xm G^T gE11 + Ym G^T gE12 + 0.25 dXc[parent])     (dY: X <-> Y, gmu1 -> gmu2)
+// G^T, the adjoint of the valid blur, is the full-size correlation with the same (symmetric) taps.  The pool term is the
+// adjoint of ms_ssim_pool: every pixel of a 2x2 cell gets a quarter of the gradient of its pooled value.
+// One CTA owns a kTH x kTW tile of one (image, channel) plane and writes each of its pixels once (no atomics: the result
+// does not depend on scheduling).  The moments are recomputed for the kFH x kFW valid positions whose window touches the
+// tile, from the masked X, Y staged with a 10-pixel apron on every side.
+constexpr int kBH = kTH + 2 * kApron, kBW = kTW + 2 * kApron, kBP = kBW + 1;   // staged input 36 x 52
+constexpr int kFH = kTH + kApron, kFW = kTW + kApron, kFP = kFW + 1;            // gradient fields 26 x 42
+constexpr int kBwdSmemFloats = 2 * kBH * kBP + 5 * kFH * kBP + 4 * kFH * kFP;
+static_assert(4 * kTH * kFP <= 5 * kFH * kBP, "the transposed H blur reuses the moment buffer");
+
+template <bool DX, bool DY>
+__global__ void __launch_bounds__(256)
+ms_ssim_level_bwd_kernel(const float* __restrict__ X, const float* __restrict__ Y, const float* __restrict__ mask, int C,
+                         int H, int W, Level k, Gauss g, const float* __restrict__ grad, const float* __restrict__ counts,
+                         const float* __restrict__ dXc, const float* __restrict__ dYc, float* __restrict__ dX,
+                         float* __restrict__ dY) {
+    extern __shared__ float smem[];
+    float(*sx)[kBP] = reinterpret_cast<float(*)[kBP]>(smem);
+    float(*sy)[kBP] = reinterpret_cast<float(*)[kBP]>(smem + kBH * kBP);
+    float(*v)[kFH][kBP] = reinterpret_cast<float(*)[kFH][kBP]>(smem + 2 * kBH * kBP);              // moments after the H blur
+    float(*f)[kFH][kFP] = reinterpret_cast<float(*)[kFH][kFP]>(smem + 2 * kBH * kBP + 5 * kFH * kBP);   // gE11 gE12 gmu1 gmu2
+    float(*t)[kTH][kFP] = reinterpret_cast<float(*)[kTH][kFP]>(smem + 2 * kBH * kBP);              // fields after G^T along H
+    const int oh = H - kApron, ow = W - kApron;
+    const int tiles_x = (W + kTW - 1) / kTW;
+    const int tx = blockIdx.x % tiles_x, ty = blockIdx.x / tiles_x;
+    const int c = blockIdx.y, b = blockIdx.z;
+    const int y0 = ty * kTH, x0 = tx * kTW;
+    const int64_t plane = (int64_t(b) * C + c) * H * W;
+    const float* mp = mask + int64_t(b) * H * W;
+    for (int i = threadIdx.x; i < kBH * kBW; i += 256) {
+        const int r = i / kBW, q = i % kBW, yy = y0 - kApron + r, xx = x0 - kApron + q;
+        float a = 0.f, d = 0.f;
+        if (yy >= 0 && yy < H && xx >= 0 && xx < W) {
+            const int64_t o = int64_t(yy) * W + xx;
+            if (mp[o] > 0.f) {
+                a = X[plane + o];
+                d = Y[plane + o];
+            }
+        }
+        sx[r][q] = a;
+        sy[r][q] = d;
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < kFH * kBW; i += 256) {
+        const int r = i / kBW, q = i % kBW;
+        float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f, a4 = 0.f;
+#pragma unroll
+        for (int j = 0; j < kWin; ++j) {
+            const float a = sx[r + j][q], d = sy[r + j][q], w = g.w[j];
+            a0 = fmaf(w, a, a0);
+            a1 = fmaf(w, d, a1);
+            a2 = fmaf(w, a * a, a2);
+            a3 = fmaf(w, d * d, a3);
+            a4 = fmaf(w, a * d, a4);
+        }
+        v[0][r][q] = a0; v[1][r][q] = a1; v[2][r][q] = a2; v[3][r][q] = a3; v[4][r][q] = a4;
+    }
+    __syncthreads();
+    const float nb = counts[b] + 1e-10f;
+    const float ws = grad[(int64_t(b) * C + c) * 2] / nb, wc = grad[(int64_t(b) * C + c) * 2 + 1] / nb;
+    for (int i = threadIdx.x; i < kFH * kFW; i += 256) {
+        const int r = i / kFW, q = i % kFW, yy = y0 - kApron + r, xx = x0 - kApron + q;
+        float e11 = 0.f, e12 = 0.f, gm1 = 0.f, gm2 = 0.f;
+        if (yy >= 0 && yy < oh && xx >= 0 && xx < ow && counted(mp, yy, xx, H, W, k.scale_h, k.scale_w)) {
+            float m[5] = {0.f, 0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+            for (int j = 0; j < kWin; ++j) {
+                const float w = g.w[j];
+#pragma unroll
+                for (int e = 0; e < 5; ++e) m[e] = fmaf(w, v[e][r][q + j], m[e]);
+            }
+            const float mu1 = m[0], mu2 = m[1];
+            const float s1 = m[2] - mu1 * mu1, s2 = m[3] - mu2 * mu2, s12 = m[4] - mu1 * mu2;
+            const float B1 = mu1 * mu1 + mu2 * mu2 + k.C1, B2 = s1 + s2 + k.C2;
+            const float l = (2.f * mu1 * mu2 + k.C1) / B1, cs = (2.f * s12 + k.C2) / B2;
+            const float g_cs = ws * l + wc, g_l = ws * cs;
+            e11 = -g_cs * cs / B2;
+            e12 = 2.f * g_cs / B2;
+            if (DX) gm1 = 2.f * g_l * (mu2 - l * mu1) / B1 - 2.f * mu1 * e11 - mu2 * e12;
+            if (DY) gm2 = 2.f * g_l * (mu1 - l * mu2) / B1 - 2.f * mu2 * e11 - mu1 * e12;
+        }
+        f[0][r][q] = e11;
+        f[1][r][q] = e12;
+        if (DX) f[2][r][q] = gm1;
+        if (DY) f[3][r][q] = gm2;
+    }
+    __syncthreads();
+    // G^T along H: output row r of the tile gathers the field rows r .. r + 10 (taps mirrored = the same taps)
+    for (int i = threadIdx.x; i < kTH * kFW; i += 256) {
+        const int r = i / kFW, q = i % kFW;
+        float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
+#pragma unroll
+        for (int j = 0; j < kWin; ++j) {
+            const float w = g.w[j];
+            a0 = fmaf(w, f[0][r + j][q], a0);
+            a1 = fmaf(w, f[1][r + j][q], a1);
+            if (DX) a2 = fmaf(w, f[2][r + j][q], a2);
+            if (DY) a3 = fmaf(w, f[3][r + j][q], a3);
+        }
+        t[0][r][q] = a0;
+        t[1][r][q] = a1;
+        if (DX) t[2][r][q] = a2;
+        if (DY) t[3][r][q] = a3;
+    }
+    __syncthreads();
+    const int Hp = (H + 2 * (H % 2) - 2) / 2 + 1, Wp = (W + 2 * (W % 2) - 2) / 2 + 1;
+    for (int i = threadIdx.x; i < kTH * kTW; i += 256) {
+        const int r = i / kTW, q = i % kTW, yy = y0 + r, xx = x0 + q;
+        if (yy >= H || xx >= W) continue;
+        float o11 = 0.f, o12 = 0.f, om1 = 0.f, om2 = 0.f;
+#pragma unroll
+        for (int j = 0; j < kWin; ++j) {
+            const float w = g.w[j];
+            o11 = fmaf(w, t[0][r][q + j], o11);
+            o12 = fmaf(w, t[1][r][q + j], o12);
+            if (DX) om1 = fmaf(w, t[2][r][q + j], om1);
+            if (DY) om2 = fmaf(w, t[3][r][q + j], om2);
+        }
+        const float xm = sx[r + kApron][q + kApron], ym = sy[r + kApron][q + kApron];
+        const int64_t o = int64_t(yy) * W + xx;
+        const bool in = mp[o] > 0.f;
+        const int64_t po = ((int64_t(b) * C + c) * Hp + (yy + H % 2) / 2) * Wp + (xx + W % 2) / 2;   // parent in the pool
+        if (DX) {
+            float d = om1 + 2.f * xm * o11 + ym * o12;
+            if (dXc) d += 0.25f * dXc[po];
+            dX[plane + o] = in ? d : 0.f;
+        }
+        if (DY) {
+            float d = om2 + 2.f * ym * o11 + xm * o12;
+            if (dYc) d += 0.25f * dYc[po];
+            dY[plane + o] = in ? d : 0.f;
+        }
+    }
+}
+
+template <bool DX, bool DY>
+int launch_level_bwd(const float* X, const float* Y, const float* mask, int B, int C, int H, int W, float data_range,
+                     const float* grad, const float* counts, const float* dXc, const float* dYc, float* dX, float* dY,
+                     cudaStream_t st) {
+    constexpr int smem = kBwdSmemFloats * int(sizeof(float));
+    MWA_TRY_CUDA(cudaFuncSetAttribute(ms_ssim_level_bwd_kernel<DX, DY>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem),
+                 "ms_ssim_level_backward(smem)");
+    dim3 grid(unsigned(((W + kTW - 1) / kTW) * ((H + kTH - 1) / kTH)), unsigned(C), unsigned(B));
+    ms_ssim_level_bwd_kernel<DX, DY><<<grid, 256, smem, st>>>(X, Y, mask, C, H, W, level_consts(H, W, data_range),
+                                                             gauss_taps(), grad, counts, dXc, dYc, dX, dY);
+    return check_launch("ms_ssim_level_backward");
+}
+
 }  // namespace
 }  // namespace b200
 
@@ -165,21 +352,10 @@ int ms_ssim_level_forward(const float* X, const float* Y, const float* mask, int
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     MWA_TRY_CUDA(cudaMemsetAsync(sums, 0, sizeof(float) * 2 * B * C, st), "ms_ssim_level(memset)");
     MWA_TRY_CUDA(cudaMemsetAsync(counts, 0, sizeof(float) * B, st), "ms_ssim_level(memset)");
-    Gauss g;
-    {
-        // metrics/masked_ms_ssim_torch.py:13-24 (_fspecial_gauss_1d) in fp32
-        float s = 0.f;
-        for (int i = 0; i < kWin; ++i) {
-            const float c = float(i - kWin / 2);
-            g.w[i] = expf(-(c * c) / (2.f * 1.5f * 1.5f));
-            s += g.w[i];
-        }
-        for (int i = 0; i < kWin; ++i) g.w[i] /= s;
-    }
     const int oh = H - kApron, ow = W - kApron;
-    const float C1 = (0.01f * data_range) * (0.01f * data_range), C2 = (0.03f * data_range) * (0.03f * data_range);
+    const Level k = level_consts(H, W, data_range);
     dim3 grid(unsigned(((ow + kTW - 1) / kTW) * ((oh + kTH - 1) / kTH)), unsigned(C), unsigned(B));
-    ms_ssim_level_kernel<<<grid, 256, 0, st>>>(X, Y, mask, C, H, W, C1, C2, float(double(H) / oh), float(double(W) / ow), g, sums,
+    ms_ssim_level_kernel<<<grid, 256, 0, st>>>(X, Y, mask, C, H, W, k.C1, k.C2, k.scale_h, k.scale_w, gauss_taps(), sums,
                                               counts);
     return check_launch("ms_ssim_level_forward");
 }
@@ -194,6 +370,19 @@ int ms_ssim_pool_forward(const float* X, const float* Y, const float* mask, int 
     if (blocks > kNumSMs * 8) blocks = kNumSMs * 8;
     ms_ssim_pool_kernel<<<unsigned(blocks), 256, 0, static_cast<cudaStream_t>(stream)>>>(X, Y, mask, C, H, W, Hp, Wp, Xo, Yo, Mo, n);
     return check_launch("ms_ssim_pool_forward");
+}
+
+int ms_ssim_level_backward(const float* X, const float* Y, const float* mask, int B, int C, int H, int W, float data_range,
+                           const float* grad, const float* counts, const float* dXc, const float* dYc, float* dX, float* dY,
+                           void* stream) {
+    if (!X || !Y || !mask || !grad || !counts || B < 0 || C <= 0) return MWA_ERR_INVALID;
+    if (H < kWin || W < kWin) return MWA_ERR_UNSUPPORTED;
+    if (B == 0) return MWA_OK;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (dX && dY) return launch_level_bwd<true, true>(X, Y, mask, B, C, H, W, data_range, grad, counts, dXc, dYc, dX, dY, st);
+    if (dX) return launch_level_bwd<true, false>(X, Y, mask, B, C, H, W, data_range, grad, counts, dXc, dYc, dX, dY, st);
+    if (dY) return launch_level_bwd<false, true>(X, Y, mask, B, C, H, W, data_range, grad, counts, dXc, dYc, dX, dY, st);
+    return MWA_OK;
 }
 
 }  // extern "C"

@@ -314,11 +314,20 @@ MWA_API int conv_forward_ex(const float* x, int64_t x_batch_stride, void* in_hi,
  *     whose nearest-resized mask is non-zero, counts[b] the number of such positions (both overwritten).  H, W >= 11.
  * ms_ssim_pool_forward  : the level's images times the binarised mask, and the binarised mask, through
  *     F.avg_pool2d(2, padding = size % 2): Xo, Yo (B, C, Hp, Wp), Mo (B, Hp, Wp) with Hp = (H + 2 (H % 2) - 2) / 2 + 1.
- * The five-level product (weights 0.0448 ... 0.1333, relu, mean over images and channels) is a handful of scalars. */
+ * The five-level product (weights 0.0448 ... 0.1333, relu, mean over images and channels) is a handful of scalars.
+ * ms_ssim_level_backward : the adjoint of one level of S[b,c] = sums[.., 0] / N_b and CS[b,c] = sums[.., 1] / N_b,
+ *     N_b = counts[b] + 1e-10, plus that of the pool that fed the next level.  X, Y, mask, B, C, H, W, data_range as given to
+ *     ms_ssim_level_forward, `counts` as it returned them; grad (B, C, 2) = dL/dS, dL/dCS per (b, c); dXc / dYc
+ *     (B, C, Hp, Wp) the gradients of the next level's X / Y (NULL at the coarsest level).  Writes dX / dY (B, C, H, W):
+ *     the gradient of X / Y, 0 where the mask is not > 0; either may be NULL and its work is skipped (the dX chain never
+ *     reads dYc).  Run from the coarsest level to the finest; no atomics, so the result is deterministic.  H, W >= 11. */
 MWA_API int ms_ssim_level_forward(const float* X, const float* Y, const float* mask, int B, int C, int H, int W,
                                   float data_range, float* sums, float* counts, void* stream);
 MWA_API int ms_ssim_pool_forward(const float* X, const float* Y, const float* mask, int B, int C, int H, int W, float* Xo,
                                  float* Yo, float* Mo, void* stream);
+MWA_API int ms_ssim_level_backward(const float* X, const float* Y, const float* mask, int B, int C, int H, int W,
+                                   float data_range, const float* grad, const float* counts, const float* dXc,
+                                   const float* dYc, float* dX, float* dY, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Range-ANS coder of the bitstream (HOST functions: every pointer is host memory; SURVEY.md 8f, rank 4)   replaces the
