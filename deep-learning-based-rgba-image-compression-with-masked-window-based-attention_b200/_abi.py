@@ -95,6 +95,8 @@ _SIGNATURES = {
     "mask_constraint_forward": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "rgba8_ingest": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "rgba8_egress": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
+    "rgba16_ingest": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
+    "rgba16_egress": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 

@@ -540,30 +540,50 @@ class AutoEncoder(nn.Module):
         The image is converted on the device to the planes the model was trained on (a / 255, colour premultiplied by the
         binarised alpha; csrc/rgba8.cu) and padded at the bottom and right with transparent pixels to multiples of 64, then
         compressed as `compress` does; the stream format is unchanged.  Returns {"strings", "shape", "size": (H, W)}."""
-        if coder not in ("host", "device"):
-            raise ValueError(f"coder must be 'host' or 'device' (got {coder!r})")
-        rgba8_mod.as_batch(rgba8, (4,), "rgba8")
-        image, alpha, size = rgba8_mod.rgba8_ingest(rgba8, self.entropy_bottleneck.quantiles.device)
-        out = self.compress(image, alpha, coder=coder, lanes=lanes)
-        out["size"] = size
-        return out
+        return self._compress_rgba(rgba8, torch.uint8, rgba8_mod.rgba8_ingest, coder, lanes)
 
     @torch.no_grad()
     def decompress_rgba8(self, strings, shape, alpha8):
         """decompress to uint8 (B, H, W, 4).  alpha8: uint8 (B, H, W) or (H, W), the images' alpha (the decoder takes it as
         `decompress` takes the mask); it gives the original size, and shape must be (ceil(H / 64), ceil(W / 64)).  Alpha is
         copied through; RGB = rint(clamp(x_hat, 0, 1) * 255) where alpha > 0, else 0, cropped to H x W in one launch."""
-        a8 = rgba8_mod.as_batch(alpha8.unsqueeze(-1) if isinstance(alpha8, torch.Tensor) else alpha8, (1,), "alpha8")
-        B, H, W, _ = a8.shape
+        return self._decompress_rgba(strings, shape, alpha8, torch.uint8, rgba8_mod.rgba8_ingest, rgba8_mod.rgba8_egress)
+
+    @torch.no_grad()
+    def compress_rgba16(self, rgba16, coder="host", lanes=None):
+        """compress_rgba8 for 16-bit RGBA: uint16 (B, H, W, 4) or (H, W, 4), converted with full scale 65535.  The stream
+        format is the same: for 8-bit values v, rgba16 = 257 * v gives exactly compress_rgba8's strings."""
+        return self._compress_rgba(rgba16, torch.uint16, rgba8_mod.rgba16_ingest, coder, lanes)
+
+    @torch.no_grad()
+    def decompress_rgba16(self, strings, shape, alpha16):
+        """decompress_rgba8 to uint16 (B, H, W, 4) given the uint16 (B, H, W) or (H, W) alpha: RGB = rint(clamp(x_hat, 0, 1)
+        * 65535) where alpha > 0, else 0.  Strings from compress_rgba8, compress_rgba16 or compress decode alike."""
+        return self._decompress_rgba(strings, shape, alpha16, torch.uint16, rgba8_mod.rgba16_ingest,
+                                     rgba8_mod.rgba16_egress)
+
+    def _compress_rgba(self, rgba, dtype, ingest, coder, lanes):
+        if coder not in ("host", "device"):
+            raise ValueError(f"coder must be 'host' or 'device' (got {coder!r})")
+        rgba8_mod.as_batch(rgba, (4,), f"rgba{8 * dtype.itemsize}", dtype)
+        image, alpha, size = ingest(rgba, self.entropy_bottleneck.quantiles.device)
+        out = self.compress(image, alpha, coder=coder, lanes=lanes)
+        out["size"] = size
+        return out
+
+    def _decompress_rgba(self, strings, shape, alpha_in, dtype, ingest, egress):
+        a = rgba8_mod.as_batch(alpha_in.unsqueeze(-1) if isinstance(alpha_in, torch.Tensor) else alpha_in, (1,),
+                               f"alpha{8 * dtype.itemsize}", dtype)
+        B, H, W, _ = a.shape
         want = (rgba8_mod.padded(H) // rgba8_mod.PAD, rgba8_mod.padded(W) // rgba8_mod.PAD)
         if tuple(int(v) for v in shape) != want:
             raise ValueError(f"shape {tuple(shape)} does not fit a {H} x {W} alpha: expected {want}")
         if len(strings) != 2 or len(strings[0]) != B or len(strings[1]) != B:
             raise ValueError(f"expected [y strings, z strings] of {B} images each")
-        a8 = rgba8_mod.on_device(a8, self.entropy_bottleneck.quantiles.device)
-        _, alpha, _ = rgba8_mod.rgba8_ingest(a8)
+        a = rgba8_mod.on_device(a, self.entropy_bottleneck.quantiles.device)
+        _, alpha, _ = ingest(a)
         x_hat, streams = self._decode(strings, shape, alpha)
-        out = rgba8_mod.rgba8_egress(x_hat, a8.view(B, H, W))
+        out = egress(x_hat, a.view(B, H, W))
         if streams is not None:
             streams.check()
         return out

@@ -1,12 +1,13 @@
-"""8-bit RGBA images of any size in and out of the codec (csrc/rgba8.cu, DESIGN.md 4.8).
+"""8- and 16-bit RGBA images of any size in and out of the codec (csrc/rgba8.cu, DESIGN.md 4.8).
 
-    rgba8_ingest(rgba8)          uint8 (B, H, W, 4) or (H, W, 4) -> fp32 image (B, 3, Hp, Wp), alpha (B, 1, Hp, Wp), (H, W)
-                                 uint8 (..., 1) (alpha only)     -> None, alpha, (H, W)
-    rgba8_egress(x_hat, alpha8)  fp32 (B, 3, Hp, Wp) + uint8 (B, H, W) -> uint8 (B, H, W, 4) on x_hat's device
+    rgba8_ingest(rgba8)            uint8 (B, H, W, 4) or (H, W, 4) -> fp32 image (B, 3, Hp, Wp), alpha (B, 1, Hp, Wp), (H, W)
+                                   uint8 (..., 1) (alpha only)     -> None, alpha, (H, W)
+    rgba8_egress(x_hat, alpha8)    fp32 (B, 3, Hp, Wp) + uint8 (B, H, W) -> uint8 (B, H, W, 4) on x_hat's device
+    rgba16_ingest / rgba16_egress  the same for uint16 samples, full scale 65535
 
 Hp / Wp are H / W rounded up to a multiple of 64 (the model's coarsest stride: z is Hp / 64 x Wp / 64); the padding, at the
-bottom and right, is transparent.  The planes are what the model was trained on: a / 255 and the colour premultiplied by
-the binarised alpha.  One kernel launch each way.
+bottom and right, is transparent.  The planes are what the model was trained on: a / full scale and the colour
+premultiplied by the binarised alpha.  One kernel launch each way.
 """
 from __future__ import annotations
 
@@ -37,16 +38,20 @@ def on_device(t: torch.Tensor, device) -> torch.Tensor:
         return t
     device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
     if device.type != "cuda":
-        raise _abi.MwaB200Error(f"8-bit images are converted on a CUDA device (got {device}); there is no CPU fallback")
+        raise _abi.MwaB200Error(f"RGBA images are converted on a CUDA device (got {device}); there is no CPU fallback")
     return t.to(device, non_blocking=t.is_pinned())
 
 
-def as_batch(t: torch.Tensor, channels: tuple, what: str) -> torch.Tensor:
-    """uint8 (B, H, W, C) or (H, W, C) with C in `channels`, contiguous, as (B, H, W, C)"""
+def _name(dtype: torch.dtype) -> str:
+    return str(dtype).removeprefix("torch.")
+
+
+def as_batch(t: torch.Tensor, channels: tuple, what: str, dtype: torch.dtype = torch.uint8) -> torch.Tensor:
+    """`dtype` (B, H, W, C) or (H, W, C) with C in `channels`, contiguous, as (B, H, W, C)"""
     if not isinstance(t, torch.Tensor):
         raise ValueError(f"{what} must be a torch.Tensor (got {type(t).__name__})")
-    if t.dtype != torch.uint8:
-        raise _abi.MwaB200Error(f"{what} must be uint8 (got {t.dtype})")
+    if t.dtype != dtype:
+        raise _abi.MwaB200Error(f"{what} must be {_name(dtype)} (got {t.dtype})")
     if t.dim() not in (3, 4) or t.shape[-1] not in channels:
         raise ValueError(f"{what} must be (B, H, W, C) or (H, W, C) with C in {channels} (got {tuple(t.shape)})")
     if not t.is_contiguous():
@@ -54,45 +59,66 @@ def as_batch(t: torch.Tensor, channels: tuple, what: str) -> torch.Tensor:
     return t if t.dim() == 4 else t.unsqueeze(0)
 
 
-def rgba8_ingest(rgba8: torch.Tensor, device=None):
-    """(image, alpha, (H, W)): the fp32 planes of uint8 RGBA (C = 4; image None for C = 1, an alpha plane alone), padded to
-    multiples of 64.  A CPU input is copied to `device` (default: the current CUDA device) once."""
-    t = as_batch(rgba8, (1, 4), "rgba8")
+def _ingest(t: torch.Tensor, device, dtype: torch.dtype, what: str):
+    t = as_batch(t, (1, 4), what, dtype)
     B, H, W, C = t.shape
     _check_size(B, H, W)
     t = on_device(t, device)
-    if t.data_ptr() % 4:
+    if t.data_ptr() % (4 * t.element_size()):       # whole Words (one RGBA pixel, or 4 alpha samples) for the kernel
         t = t.clone()
     Hp, Wp = padded(H), padded(W)
     alpha = torch.empty(B, 1, Hp, Wp, dtype=torch.float32, device=t.device)
     image = torch.empty(B, 3, Hp, Wp, dtype=torch.float32, device=t.device) if C == 4 else None
     lib = _abi.load()
     with torch.cuda.device(t.device):
-        _abi.check(lib.rgba8_ingest(t.data_ptr(), _abi.ptr(image), alpha.data_ptr(), B, H, W, C, _abi.stream_handle()),
-                   "rgba8_ingest")
+        _abi.check(getattr(lib, what + "_ingest")(t.data_ptr(), _abi.ptr(image), alpha.data_ptr(), B, H, W, C,
+                                                  _abi.stream_handle()), what + "_ingest")
     _abi.count_launches(1)
     return image, alpha, (H, W)
+
+
+def _egress(x_hat: torch.Tensor, alpha_in: torch.Tensor, dtype: torch.dtype, what: str) -> torch.Tensor:
+    _abi.require_cuda_f32(x_hat, "x_hat")
+    name = "alpha" + what.removeprefix("rgba")
+    if alpha_in.dtype != dtype or alpha_in.dim() != 3 or not alpha_in.is_contiguous():
+        raise ValueError(f"{name} must be contiguous {_name(dtype)} (B, H, W) (got {alpha_in.dtype} {tuple(alpha_in.shape)})")
+    B, H, W = alpha_in.shape
+    _check_size(B, H, W)
+    if tuple(x_hat.shape) != (B, 3, padded(H), padded(W)):
+        raise ValueError(f"x_hat must be (B, 3, Hp, Wp) = {(B, 3, padded(H), padded(W))} for alpha {tuple(alpha_in.shape)} "
+                         f"(got {tuple(x_hat.shape)})")
+    alpha_in = on_device(alpha_in, x_hat.device)
+    x_hat = x_hat.contiguous()
+    if x_hat.data_ptr() % 16:
+        x_hat = x_hat.clone()
+    out = torch.empty(B, H, W, 4, dtype=dtype, device=x_hat.device)
+    lib = _abi.load()
+    with torch.cuda.device(x_hat.device):
+        _abi.check(getattr(lib, what + "_egress")(x_hat.data_ptr(), alpha_in.data_ptr(), out.data_ptr(), B, H, W,
+                                                  _abi.stream_handle()), what + "_egress")
+    _abi.count_launches(1)
+    return out
+
+
+def rgba8_ingest(rgba8: torch.Tensor, device=None):
+    """(image, alpha, (H, W)): the fp32 planes of uint8 RGBA (C = 4; image None for C = 1, an alpha plane alone), padded to
+    multiples of 64.  A CPU input is copied to `device` (default: the current CUDA device) once."""
+    return _ingest(rgba8, device, torch.uint8, "rgba8")
 
 
 def rgba8_egress(x_hat: torch.Tensor, alpha8: torch.Tensor) -> torch.Tensor:
     """uint8 (B, H, W, 4) from the decoder's fp32 (B, 3, Hp, Wp) x_hat (unclamped) and the uint8 (B, H, W) alpha: A = alpha,
     RGB = rint(clamp(x_hat, 0, 1) * 255) where alpha > 0, else 0"""
-    _abi.require_cuda_f32(x_hat, "x_hat")
-    if alpha8.dtype != torch.uint8 or alpha8.dim() != 3 or not alpha8.is_contiguous():
-        raise ValueError(f"alpha8 must be contiguous uint8 (B, H, W) (got {alpha8.dtype} {tuple(alpha8.shape)})")
-    B, H, W = alpha8.shape
-    _check_size(B, H, W)
-    if tuple(x_hat.shape) != (B, 3, padded(H), padded(W)):
-        raise ValueError(f"x_hat must be (B, 3, Hp, Wp) = {(B, 3, padded(H), padded(W))} for alpha {tuple(alpha8.shape)} "
-                         f"(got {tuple(x_hat.shape)})")
-    alpha8 = on_device(alpha8, x_hat.device)
-    x_hat = x_hat.contiguous()
-    if x_hat.data_ptr() % 16:
-        x_hat = x_hat.clone()
-    out = torch.empty(B, H, W, 4, dtype=torch.uint8, device=x_hat.device)
-    lib = _abi.load()
-    with torch.cuda.device(x_hat.device):
-        _abi.check(lib.rgba8_egress(x_hat.data_ptr(), alpha8.data_ptr(), out.data_ptr(), B, H, W, _abi.stream_handle()),
-                   "rgba8_egress")
-    _abi.count_launches(1)
-    return out
+    return _egress(x_hat, alpha8, torch.uint8, "rgba8")
+
+
+def rgba16_ingest(rgba16: torch.Tensor, device=None):
+    """rgba8_ingest for uint16 samples: alpha = a / 65535, colour / 65535 premultiplied by the binarised alpha.  For 8-bit
+    values v, rgba16 = 257 * v gives exactly rgba8_ingest's planes."""
+    return _ingest(rgba16, device, torch.uint16, "rgba16")
+
+
+def rgba16_egress(x_hat: torch.Tensor, alpha16: torch.Tensor) -> torch.Tensor:
+    """uint16 (B, H, W, 4) from the decoder's fp32 (B, 3, Hp, Wp) x_hat (unclamped) and the uint16 (B, H, W) alpha:
+    A = alpha, RGB = rint(clamp(x_hat, 0, 1) * 65535) where alpha > 0, else 0"""
+    return _egress(x_hat, alpha16, torch.uint16, "rgba16")

@@ -412,6 +412,26 @@ MWA_API int rate_forward(const float* input, const float* x_hat, const float* ma
 MWA_API int rgba8_ingest(const uint8_t* rgba8, float* image, float* alpha, int B, int H, int W, int C, void* stream);
 MWA_API int rgba8_egress(const float* x_hat, const uint8_t* alpha8, uint8_t* rgba8, int B, int H, int W, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * 16-bit RGBA images of any size (csrc/rgba8.cu; DESIGN.md 4.8)   the same conversion, padding and status codes as the
+ *   8-bit pair for uint16 samples (PNG-16, 16-bit TIFF), with full scale 65535.
+ * rgba16_ingest : rgba16 uint16 (B, H, W, C) contiguous, C = 4 (RGBA) or 1 (alpha only) -> alpha fp32 (B, 1, Hp, Wp) and,
+ *                 for C = 4, image fp32 (B, 3, Hp, Wp) (image may be NULL for C = 1).  For y < H, x < W:
+ *                   alpha = a / 65535;   image_c = rgb_c / 65535 if a > 0, else 0      (IEEE round-to-nearest divisions)
+ *                 every other element (bottom and right padding) is +0.0: transparent.  For 8-bit samples v,
+ *                 rgba16 = 257 * v gives the planes rgba8_ingest gives for v, bit for bit.
+ * rgba16_egress : x_hat fp32 (B, 3, Hp, Wp), alpha16 uint16 (B, H, W) -> rgba16 uint16 (B, H, W, 4), per pixel:
+ *                   A = alpha16;   RGB = rint(clamp(x_hat, 0, 1) * 65535) (fp32 multiply, half to even; NaN -> 0) if A > 0,
+ *                   else 0
+ * MWA_ERR_INVALID before any CUDA call: B < 0, H < 1, W < 1, C not in {1, 4}, or B * Hp * Wp * 48 >= 2^31; then, for
+ *   B > 0, a NULL pointer.  MWA_ERR_ALIGNMENT: an fp32 plane not 16-byte aligned, an RGBA buffer not 8-byte aligned, or an
+ *   alpha-only buffer not 2-byte aligned.  B = 0 returns MWA_OK and launches nothing.  One launch each, no allocation, no
+ *   synchronisation.
+ * ------------------------------------------------------------------------------------------------ */
+MWA_API int rgba16_ingest(const uint16_t* rgba16, float* image, float* alpha, int B, int H, int W, int C, void* stream);
+MWA_API int rgba16_egress(const float* x_hat, const uint16_t* alpha16, uint16_t* rgba16, int B, int H, int W,
+                          void* stream);
+
 #ifdef __cplusplus
 }
 #endif

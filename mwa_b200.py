@@ -56,5 +56,7 @@ HostPipeline = pipeline.HostPipeline
 invalidate_param_blocks = _params.invalidate_param_blocks
 rgba8_ingest = rgba8.rgba8_ingest
 rgba8_egress = rgba8.rgba8_egress
+rgba16_ingest = rgba8.rgba16_ingest
+rgba16_egress = rgba8.rgba16_egress
 MwaB200Error = _abi.MwaB200Error
 ALGO_AUTO, ALGO_SIMT, ALGO_TCGEN05 = _abi.ALGO_AUTO, _abi.ALGO_SIMT, _abi.ALGO_TCGEN05

@@ -1,20 +1,22 @@
 #!/usr/bin/env python
-"""8-bit RGBA ingest / egress (csrc/rgba8.cu, DESIGN.md 4.8): kernel time, codec wall time against the fp32-plane calls, and
-the host-to-device copy of uint8 against fp32.
+"""8- or 16-bit RGBA ingest / egress (csrc/rgba8.cu, DESIGN.md 4.8): kernel time, codec wall time against the fp32-plane
+calls, and the host-to-device copy of uint8 / uint16 against fp32.
 
-    python tools/rgba8_time.py --out DIR [--launches 50] [--reps 5]
+    python tools/rgba8_time.py --out DIR [--bits 8|16] [--launches 50] [--reps 5]
 
 Reports, with the GPU's name and power limit read in the same run:
-  * kernel time of rgba8_ingest (RGBA and alpha-only) and rgba8_egress at batch 16 x 768x512 (bench.py's workload) and at
+  * kernel time of rgba{bits}_ingest (RGBA and alpha-only) and rgba{bits}_egress at batch 16 x 768x512 (bench.py's
+    workload) and at
     batch 1 x 2160x3840: CUDA events around each of --launches launches, a 512 MiB buffer written between launches so that
-    no launch finds its data in the 126 MB L2; algorithmic bytes per launch (uint8 read / written + fp32 planes read /
-    written, the egress reading only the H x W crop of x_hat) and GB/s, against the data-sheet HBM peak (7.7 TB/s, HGX B200
-    per GPU) and against a device-to-device copy measured in the same run;
+    no launch finds its data in the 126 MB L2; algorithmic bytes per launch (integer samples read / written + fp32 planes
+    read / written, the egress reading only the H x W crop of x_hat) and GB/s, against the data-sheet HBM peak (7.7 TB/s,
+    HGX B200 per GPU) and against a device-to-device copy measured in the same run;
   * wall time (median of --reps runs after a warm-up, each ending in a device synchronise) of compress_rgba8 /
-    decompress_rgba8 and of compress / decompress on the same fp32 planes, host and device coder, bench workload, RGBACodec
-    random init under torch.manual_seed(234);
-  * host-to-device copy of the bench batch from pinned memory: uint8 (B, H, W, 4) against fp32 (B, 4, H, W).
-Writes DIR/rgba8_time.json and prints the same JSON.
+    decompress_rgba8 (and, with --bits 16, compress_rgba16 / decompress_rgba16 on 257 times the same bytes) and of
+    compress / decompress on the same fp32 planes, host and device coder, bench workload, RGBACodec random init under
+    torch.manual_seed(234);
+  * host-to-device copy of the bench batch from pinned memory: uint8 / uint16 (B, H, W, 4) against fp32 (B, 4, H, W).
+Writes DIR/rgba{bits}_time.json and prints the same JSON.
 """
 from __future__ import annotations
 
@@ -69,14 +71,17 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--launches", type=int, default=50)
     ap.add_argument("--reps", type=int, default=5)
-    ap.add_argument("--out", required=True, help="directory for rgba8_time.json")
+    ap.add_argument("--bits", type=int, choices=(8, 16), default=8, help="sample depth of the timed kernels")
+    ap.add_argument("--out", required=True, help="directory for rgba{bits}_time.json")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         sys.exit("rgba8_time.py measures on a CUDA device; none found")
     dev = torch.device("cuda:0")
     torch.backends.cudnn.allow_tf32 = False
     torch.backends.cuda.matmul.allow_tf32 = False
-    res = {"gpu": gpu_info(), "hbm_peak": f"{HBM_PEAK_GBPS:.0f} GB/s (NVIDIA HGX B200 data sheet, per GPU)"}
+    bits, sb = args.bits, args.bits // 8                                        # sample bytes
+    ingest, egress = getattr(mwa_b200, f"rgba{bits}_ingest"), getattr(mwa_b200, f"rgba{bits}_egress")
+    res = {"gpu": gpu_info(), "bits": bits, "hbm_peak": f"{HBM_PEAK_GBPS:.0f} GB/s (NVIDIA HGX B200 data sheet, per GPU)"}
     flush = torch.zeros(128 * 2 ** 20, dtype=torch.float32, device=dev)            # 512 MiB
 
     # device-to-device copy in the same run: the rate an HBM-bound pass of this size can reach here
@@ -91,18 +96,21 @@ def main():
     for name, (B, H, W) in {"bench_16x768x512": (bench.BATCH_PER_GPU, bench.IMG_H, bench.IMG_W),
                             "1x3840x2160": (1, 2160, 3840)}.items():
         g = torch.Generator(device=dev).manual_seed(1)
-        rgba = torch.randint(0, 256, (B, H, W, 4), generator=g, device=dev, dtype=torch.uint8)
-        a8 = rgba[..., 3].contiguous()
+        if bits == 8:
+            rgba = torch.randint(0, 256, (B, H, W, 4), generator=g, device=dev, dtype=torch.uint8)
+        else:                                   # uniform 16-bit patterns, drawn as int16 (uint16 has no CUDA randint)
+            rgba = torch.randint(-2 ** 15, 2 ** 15, (B, H, W, 4), generator=g, device=dev, dtype=torch.int16).view(torch.uint16)
+        a8 = rgba[..., 3].contiguous() if bits == 8 else rgba.view(torch.int16)[..., 3].contiguous().view(torch.uint16)
         Hp, Wp = padded(H), padded(W)
         x_hat = torch.rand(B, 3, Hp, Wp, generator=g, device=dev)
         px, ppx = B * H * W, B * Hp * Wp
         k = {"B": B, "H": H, "W": W, "Hp": Hp, "Wp": Wp}
-        k["ingest_rgba"] = summary(event_times(lambda: mwa_b200.rgba8_ingest(rgba), args.launches, flush),
-                                   4 * px + 4 * 4 * ppx, copy_gbps)
-        k["ingest_alpha"] = summary(event_times(lambda: mwa_b200.rgba8_ingest(a8[..., None]), args.launches, flush),
-                                    px + 4 * ppx, copy_gbps)
-        k["egress"] = summary(event_times(lambda: mwa_b200.rgba8_egress(x_hat, a8), args.launches, flush),
-                              3 * 4 * px + px + 4 * px, copy_gbps)
+        k["ingest_rgba"] = summary(event_times(lambda: ingest(rgba), args.launches, flush),
+                                   4 * sb * px + 4 * 4 * ppx, copy_gbps)
+        k["ingest_alpha"] = summary(event_times(lambda: ingest(a8[..., None]), args.launches, flush),
+                                    sb * px + 4 * ppx, copy_gbps)
+        k["egress"] = summary(event_times(lambda: egress(x_hat, a8), args.launches, flush),
+                              3 * 4 * px + sb * px + 4 * sb * px, copy_gbps)
         kernels[name] = k
         del rgba, a8, x_hat
     res["kernels"] = kernels
@@ -113,37 +121,49 @@ def main():
     net = mwa_b200.RGBACodec().eval().to(dev)
     planes = bench.synthetic_rgba(bench.BATCH_PER_GPU, seed0=0)
     rgba8 = (planes.permute(0, 2, 3, 1) * 255).round().to(torch.uint8).contiguous()
-    rgba8_dev = rgba8.to(dev)
-    image, alpha, _ = mwa_b200.rgba8_ingest(rgba8_dev)           # the same planes compress_rgba8 codes
-    a8 = rgba8_dev[..., 3].contiguous()
-    wall = {"workload": f"batch {bench.BATCH_PER_GPU}, {bench.IMG_W}x{bench.IMG_H}, bench.synthetic_rgba(seed0=0) as uint8, "
-                        "RGBACodec random init (torch.manual_seed(234)), inputs on the device"}
+    depths = {8: rgba8}
+    if bits == 16:
+        depths[16] = (rgba8.to(torch.int32) * 257).to(torch.uint16)       # the same planes at 16 bits (DESIGN.md 4.8)
+    on_dev = {d: t.to(dev) for d, t in depths.items()}
+    alphas = {d: t[..., 3].contiguous().to(dev) for d, t in depths.items()}
+    image, alpha, _ = mwa_b200.rgba8_ingest(on_dev[8])            # the same planes compress_rgba8 codes
+    wall = {"workload": f"batch {bench.BATCH_PER_GPU}, {bench.IMG_W}x{bench.IMG_H}, bench.synthetic_rgba(seed0=0) as uint8"
+                        f"{' (and 257 times it as uint16)' if bits == 16 else ''}, RGBACodec random init "
+                        "(torch.manual_seed(234)), inputs on the device"}
     with torch.no_grad():
         for coder in ("host", "device"):
             r = {}
-            out8 = net.compress_rgba8(rgba8_dev, coder=coder)
+            comp = {d: getattr(net, f"compress_rgba{d}") for d in depths}
+            decomp = {d: getattr(net, f"decompress_rgba{d}") for d in depths}
             out = net.compress(image, alpha, coder=coder)
-            net.decompress_rgba8(out8["strings"], out8["shape"], a8)
             net.decompress(out["strings"], out["shape"], alpha)
-            r["compress_rgba8_ms"], r["compress_rgba8_runs_ms"], out8 = timed(
-                lambda: net.compress_rgba8(rgba8_dev, coder=coder), args.reps)
+            for d in depths:
+                o = comp[d](on_dev[d], coder=coder)
+                decomp[d](o["strings"], o["shape"], alphas[d])
             r["compress_ms"], r["compress_runs_ms"], out = timed(lambda: net.compress(image, alpha, coder=coder), args.reps)
-            r["decompress_rgba8_ms"], r["decompress_rgba8_runs_ms"], rec8 = timed(
-                lambda: net.decompress_rgba8(out8["strings"], out8["shape"], a8), args.reps)
             r["decompress_ms"], r["decompress_runs_ms"], rec = timed(
                 lambda: net.decompress(out["strings"], out["shape"], alpha)["x_hat"], args.reps)
-            r["strings_equal"] = out8["strings"] == out["strings"]
-            want = (rec[:, :, :bench.IMG_H, :bench.IMG_W] * 255).round().to(torch.uint8).permute(0, 2, 3, 1)
-            r["rgb_equals_quantised_decompress"] = bool(torch.equal(rec8[..., :3], want * (a8[..., None] > 0)))
+            for d in depths:
+                r[f"compress_rgba{d}_ms"], r[f"compress_rgba{d}_runs_ms"], o = timed(
+                    lambda: comp[d](on_dev[d], coder=coder), args.reps)
+                r[f"decompress_rgba{d}_ms"], r[f"decompress_rgba{d}_runs_ms"], rec_d = timed(
+                    lambda: decomp[d](o["strings"], o["shape"], alphas[d]), args.reps)
+                suffix = "" if d == 8 else f"_rgba{d}"
+                r["strings_equal" + suffix] = o["strings"] == out["strings"]
+                # compared on the CPU in int32: torch has no CUDA comparison for uint16
+                want = (rec[:, :, :bench.IMG_H, :bench.IMG_W] * (2 ** d - 1)).round().to(torch.int32).permute(0, 2, 3, 1)
+                got = rec_d[..., :3].cpu().to(torch.int32)
+                opaque = alphas[d].cpu().to(torch.int32)[..., None] > 0
+                r[f"rgb_equals_quantised_decompress{suffix}"] = bool(torch.equal(got, want.cpu() * opaque))
             wall[coder] = r
     res["codec_wall"] = wall
 
     # host -> device copy from pinned memory
-    h8 = rgba8.pin_memory()
+    h8 = depths[bits].pin_memory()
     h32 = planes.contiguous().pin_memory()
     d8, d32 = torch.empty_like(h8, device=dev), torch.empty_like(h32, device=dev)
     copies = {}
-    for name, (h, d) in {"uint8_BHW4": (h8, d8), "fp32_B4HW": (h32, d32)}.items():
+    for name, (h, d) in {f"uint{bits}_BHW4": (h8, d8), "fp32_B4HW": (h32, d32)}.items():
         t = event_times(lambda: d.copy_(h, non_blocking=True), 20, torch.zeros(1, device=dev))
         med = statistics.median(t)
         copies[name] = {"bytes": h.numel() * h.element_size(), "median_ms": med,
@@ -151,7 +171,7 @@ def main():
     res["h2d_pinned"] = copies
     res["gpu_after"] = gpu_info()
     os.makedirs(args.out, exist_ok=True)
-    with open(os.path.join(args.out, "rgba8_time.json"), "w") as f:
+    with open(os.path.join(args.out, f"rgba{bits}_time.json"), "w") as f:
         json.dump(res, f, indent=1)
     print(json.dumps(res))
 
