@@ -97,6 +97,10 @@ _SIGNATURES = {
     "rgba8_egress": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "rgba16_ingest": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "rgba16_egress": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
+    "rgba8_ingest_tiles": (c_int, [c_void_p, c_void_p, c_void_p] + [c_int] * 6 + [c_int64, c_int, c_void_p]),
+    "rgba8_egress_tiles": (c_int, [c_void_p, c_void_p, c_void_p] + [c_int] * 5 + [c_int64, c_int, c_void_p]),
+    "rgba16_ingest_tiles": (c_int, [c_void_p, c_void_p, c_void_p] + [c_int] * 6 + [c_int64, c_int, c_void_p]),
+    "rgba16_egress_tiles": (c_int, [c_void_p, c_void_p, c_void_p] + [c_int] * 5 + [c_int64, c_int, c_void_p]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 

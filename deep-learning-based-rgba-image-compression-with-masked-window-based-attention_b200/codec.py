@@ -540,52 +540,98 @@ class AutoEncoder(nn.Module):
         The image is converted on the device to the planes the model was trained on (a / 255, colour premultiplied by the
         binarised alpha; csrc/rgba8.cu) and padded at the bottom and right with transparent pixels to multiples of 64, then
         compressed as `compress` does; the stream format is unchanged.  Returns {"strings", "shape", "size": (H, W)}."""
-        return self._compress_rgba(rgba8, torch.uint8, rgba8_mod.rgba8_ingest, coder, lanes)
+        return self._compress_rgba(rgba8, torch.uint8, None, coder, lanes)
 
     @torch.no_grad()
     def decompress_rgba8(self, strings, shape, alpha8):
         """decompress to uint8 (B, H, W, 4).  alpha8: uint8 (B, H, W) or (H, W), the images' alpha (the decoder takes it as
         `decompress` takes the mask); it gives the original size, and shape must be (ceil(H / 64), ceil(W / 64)).  Alpha is
         copied through; RGB = rint(clamp(x_hat, 0, 1) * 255) where alpha > 0, else 0, cropped to H x W in one launch."""
-        return self._decompress_rgba(strings, shape, alpha8, torch.uint8, rgba8_mod.rgba8_ingest, rgba8_mod.rgba8_egress)
+        return self._decompress_rgba(strings, shape, alpha8, torch.uint8, False)
 
     @torch.no_grad()
     def compress_rgba16(self, rgba16, coder="host", lanes=None):
         """compress_rgba8 for 16-bit RGBA: uint16 (B, H, W, 4) or (H, W, 4), converted with full scale 65535.  The stream
         format is the same: for 8-bit values v, rgba16 = 257 * v gives exactly compress_rgba8's strings."""
-        return self._compress_rgba(rgba16, torch.uint16, rgba8_mod.rgba16_ingest, coder, lanes)
+        return self._compress_rgba(rgba16, torch.uint16, None, coder, lanes)
 
     @torch.no_grad()
     def decompress_rgba16(self, strings, shape, alpha16):
         """decompress_rgba8 to uint16 (B, H, W, 4) given the uint16 (B, H, W) or (H, W) alpha: RGB = rint(clamp(x_hat, 0, 1)
         * 65535) where alpha > 0, else 0.  Strings from compress_rgba8, compress_rgba16 or compress decode alike."""
-        return self._decompress_rgba(strings, shape, alpha16, torch.uint16, rgba8_mod.rgba16_ingest,
-                                     rgba8_mod.rgba16_egress)
+        return self._decompress_rgba(strings, shape, alpha16, torch.uint16, False)
 
-    def _compress_rgba(self, rgba, dtype, ingest, coder, lanes):
+    @torch.no_grad()
+    def compress_tiled(self, rgba, tile=4096, coder="host", lanes=None):
+        """compress uint8 or uint16 RGBA (B, H, W, 4) or (H, W, 4) of any size and any batch, on the GPU or the host
+        (copied once), as independent tiles of Th x Tw = rgba8.tile_grid(H, W, tile) (DESIGN.md 4.8): tile n = (b * ty + i)
+        * tx + j covers rows i * Th.. and columns j * Tw.. of image b, padded with transparent pixels past the image.  Each
+        tile is coded exactly as compress_rgba8 / 16 codes that crop padded to Th x Tw; the passes take as many tiles as
+        one forward can index (rgba8.chunk_tiles).  Returns {"strings": [y strings, z strings] of B * ty * tx tiles each in
+        tile order, "shape": (Th / 64, Tw / 64), "size": (H, W), "grid": (ty, tx)}.  With tile >= the padded image the grid
+        is 1 x 1 and the strings are compress_rgba8 / 16's."""
+        rgba8_mod.depth(rgba, "rgba")
+        return self._compress_rgba(rgba, rgba.dtype, tile, coder, lanes)
+
+    @torch.no_grad()
+    def decompress_tiled(self, strings, shape, alpha):
+        """decompress compress_tiled's strings (or compress_rgba8 / 16's, a 1 x 1 grid) to (B, H, W, 4) of the alpha's
+        dtype, given the images' uint8 or uint16 (B, H, W) or (H, W) alpha: the grid follows from its size and the tile
+        shape; each tile decodes as decompress_rgba8 / 16 decodes it, and the tiles are stitched into one output."""
+        rgba8_mod.depth(alpha, "alpha")
+        return self._decompress_rgba(strings, shape, alpha, alpha.dtype, True)
+
+    def _compress_rgba(self, rgba, dtype, tile, coder, lanes):
+        """compress in tiles of tile_grid(H, W, tile), or of the padded image (tile None: the size guard applies), a chunk
+        of tiles per forward pass"""
         if coder not in ("host", "device"):
             raise ValueError(f"coder must be 'host' or 'device' (got {coder!r})")
-        rgba8_mod.as_batch(rgba, (4,), f"rgba{8 * dtype.itemsize}", dtype)
-        image, alpha, size = ingest(rgba, self.entropy_bottleneck.quantiles.device)
-        out = self.compress(image, alpha, coder=coder, lanes=lanes)
-        out["size"] = size
+        t = rgba8_mod.as_batch(rgba, (4,), f"rgba{8 * dtype.itemsize}", dtype)
+        B, H, W, _ = t.shape
+        if tile is None:
+            rgba8_mod._check_size(B, H, W)
+            Th, Tw, ty, tx = rgba8_mod.padded(H), rgba8_mod.padded(W), 1, 1
+        else:
+            Th, Tw, ty, tx = rgba8_mod.tile_grid(H, W, tile)
+        t = rgba8_mod.staged(t, self.entropy_bottleneck.quantiles.device)
+        n, per = B * ty * tx, rgba8_mod.chunk_tiles(Th, Tw)
+        strings = [[], []]
+        for first in range(0, max(n, 1), per):
+            image, alpha = rgba8_mod.ingest_tiles(t, (Th, Tw), first, min(per, n - first))
+            out = self.compress(image, alpha, coder=coder, lanes=lanes)
+            strings[0] += out["strings"][0]
+            strings[1] += out["strings"][1]
+        out["strings"], out["size"] = strings, (H, W)
+        if tile is not None:
+            out["shape"], out["grid"] = (Th // rgba8_mod.PAD, Tw // rgba8_mod.PAD), (ty, tx)
         return out
 
-    def _decompress_rgba(self, strings, shape, alpha_in, dtype, ingest, egress):
+    def _decompress_rgba(self, strings, shape, alpha_in, dtype, tiled):
         a = rgba8_mod.as_batch(alpha_in.unsqueeze(-1) if isinstance(alpha_in, torch.Tensor) else alpha_in, (1,),
                                f"alpha{8 * dtype.itemsize}", dtype)
         B, H, W, _ = a.shape
         want = (rgba8_mod.padded(H) // rgba8_mod.PAD, rgba8_mod.padded(W) // rgba8_mod.PAD)
-        if tuple(int(v) for v in shape) != want:
+        if tiled:
+            Th, Tw, ty, tx = rgba8_mod.tiles_of(H, W, shape)
+        elif tuple(int(v) for v in shape) != want:
             raise ValueError(f"shape {tuple(shape)} does not fit a {H} x {W} alpha: expected {want}")
-        if len(strings) != 2 or len(strings[0]) != B or len(strings[1]) != B:
-            raise ValueError(f"expected [y strings, z strings] of {B} images each")
-        a = rgba8_mod.on_device(a, self.entropy_bottleneck.quantiles.device)
-        _, alpha, _ = ingest(a)
-        x_hat, streams = self._decode(strings, shape, alpha)
-        out = egress(x_hat, a.view(B, H, W))
-        if streams is not None:
-            streams.check()
+        else:
+            Th, Tw, ty, tx = want[0] * rgba8_mod.PAD, want[1] * rgba8_mod.PAD, 1, 1
+        n = B * ty * tx
+        if len(strings) != 2 or len(strings[0]) != n or len(strings[1]) != n:
+            raise ValueError(f"expected [y strings, z strings] of {n} {'tiles' if tiled else 'images'} each")
+        if not tiled:
+            rgba8_mod._check_size(B, H, W)
+        a = rgba8_mod.staged(a, self.entropy_bottleneck.quantiles.device)
+        out = torch.empty(B, H, W, 4, dtype=dtype, device=a.device)
+        per = rgba8_mod.chunk_tiles(Th, Tw)
+        for first in range(0, max(n, 1), per):
+            count = min(per, n - first)
+            _, alpha = rgba8_mod.ingest_tiles(a, (Th, Tw), first, count)
+            x_hat, streams = self._decode([strings[0][first:first + count], strings[1][first:first + count]], shape, alpha)
+            rgba8_mod.egress_tiles(x_hat, a.view(B, H, W), out, first)
+            if streams is not None:
+                streams.check()
         return out
 
     def detail(self, input, mask, reconmask, me2=None, me3=None):

@@ -432,6 +432,33 @@ MWA_API int rgba16_ingest(const uint16_t* rgba16, float* image, float* alpha, in
 MWA_API int rgba16_egress(const float* x_hat, const uint16_t* alpha16, uint16_t* rgba16, int B, int H, int W,
                           void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * RGBA images in independent tiles (csrc/rgba8.cu; DESIGN.md 4.8)   the same conversion, tile by tile, for images or
+ *   batches beyond what one forward pass can index.  The B images of H x W split into tiles of Th x Tw (Th, Tw positive
+ *   multiples of 64): ty = ceil(H / Th) tile rows, tx = ceil(W / Tw) tile columns per image.  Tile n = (b * ty + i) * tx + j
+ *   covers rows [i * Th, (i + 1) * Th) and columns [j * Tw, (j + 1) * Tw) of image b; its pixels outside the image are
+ *   transparent (+0.0 in every plane).  A call covers tiles [first, first + count); local tile t = n - first.
+ * rgba{8,16}_ingest_tiles : T (B, H, W, C) contiguous, C = 4 or 1 -> alpha fp32 (count, 1, Th, Tw) and, for C = 4, image
+ *                 fp32 (count, 3, Th, Tw); per pixel the rules of rgba{8,16}_ingest.
+ * rgba{8,16}_egress_tiles : x_hat fp32 (count, 3, Th, Tw), alpha T (B, H, W) -> the pixels of T (B, H, W, 4) that tiles
+ *                 [first, first + count) cover, per pixel the rules of rgba{8,16}_egress; no other byte is written.
+ *   rgba{8,16}_ingest / _egress are the case Th = Hp, Tw = Wp, first = 0, count = B.  Offsets are 64-bit: the images may
+ *   exceed 2^31 bytes; only one call's planes are bounded.
+ * MWA_ERR_INVALID before any CUDA call: B < 0, H < 1, W < 1, C not in {1, 4}, Th or Tw not a positive multiple of 64,
+ *   first < 0, count < 0, first + count > B * ty * tx, or, for count > 0, count * Th * Tw * 48 >= 2^31, ty * Th >= 2^31
+ *   or tx * Tw >= 2^31 (the last tile row or column must end within int coordinates); then, for count > 0, a NULL
+ *   pointer.  MWA_ERR_ALIGNMENT: the rules of the untiled entry points.  count = 0 returns MWA_OK and launches nothing.
+ *   One launch each, no allocation, no synchronisation.
+ * ------------------------------------------------------------------------------------------------ */
+MWA_API int rgba8_ingest_tiles(const uint8_t* rgba8, float* image, float* alpha, int B, int H, int W, int C, int Th, int Tw,
+                               int64_t first, int count, void* stream);
+MWA_API int rgba8_egress_tiles(const float* x_hat, const uint8_t* alpha8, uint8_t* rgba8, int B, int H, int W, int Th,
+                               int Tw, int64_t first, int count, void* stream);
+MWA_API int rgba16_ingest_tiles(const uint16_t* rgba16, float* image, float* alpha, int B, int H, int W, int C, int Th,
+                                int Tw, int64_t first, int count, void* stream);
+MWA_API int rgba16_egress_tiles(const float* x_hat, const uint16_t* alpha16, uint16_t* rgba16, int B, int H, int W, int Th,
+                                int Tw, int64_t first, int count, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -58,5 +58,8 @@ rgba8_ingest = rgba8.rgba8_ingest
 rgba8_egress = rgba8.rgba8_egress
 rgba16_ingest = rgba8.rgba16_ingest
 rgba16_egress = rgba8.rgba16_egress
+tile_grid = rgba8.tile_grid
+ingest_tiles = rgba8.ingest_tiles
+egress_tiles = rgba8.egress_tiles
 MwaB200Error = _abi.MwaB200Error
 ALGO_AUTO, ALGO_SIMT, ALGO_TCGEN05 = _abi.ALGO_AUTO, _abi.ALGO_SIMT, _abi.ALGO_TCGEN05

@@ -17,6 +17,20 @@ Reports, with the GPU's name and power limit read in the same run:
     torch.manual_seed(234);
   * host-to-device copy of the bench batch from pinned memory: uint8 / uint16 (B, H, W, 4) against fp32 (B, 4, H, W).
 Writes DIR/rgba{bits}_time.json and prints the same JSON.
+
+    python tools/rgba8_time.py --tiled --parent-lib PARENT.so --out DIR [--launches 50] [--reps 3]
+
+measures the tiled path instead (DESIGN.md 4.8, "Tiles") and writes DIR/rgba_tiled_time.json:
+  * the untiled kernels (rgba8 / rgba16 ingest RGBA, ingest alpha, egress) of this build against those of PARENT.so, the
+    library of the commit before the tile kernels, built into a scratch directory (e.g. `git worktree add DIR HEAD~1`, then
+    `python -c "import mwa_b200; mwa_b200.build()"` there): launches of the two alternate, one timed pair at a time, at
+    the workloads above;
+  * the tile kernels on a chunk (2 tiles of 4096 x 4096) of a 1 x 8192 x 8192 image, 8- and 16-bit, with algorithmic
+    bytes and GB/s;
+  * compress_tiled / decompress_tiled wall time at 1 x 8192 x 8192, both coders, with the chunk count and
+    torch.cuda.max_memory_allocated of each call;
+  * at 1 x 4096 x 4096, untiled against tile = 2048: string bytes and wall time.  The model is randomly initialised
+    (torch.manual_seed(234)), so the bytes show the size of the tiling overhead, not a rate the trained model reaches.
 """
 from __future__ import annotations
 
@@ -67,15 +81,182 @@ def summary(times, nbytes, copy_gbps):
             "of_measured_copy": gbps / copy_gbps}
 
 
+def random_samples(shape, bits, g, dev):
+    """uniform uint8 / uint16 samples (16-bit ones drawn as int16: uint16 has no CUDA randint)"""
+    if bits == 8:
+        return torch.randint(0, 256, shape, generator=g, device=dev, dtype=torch.uint8)
+    return torch.randint(-2 ** 15, 2 ** 15, shape, generator=g, device=dev, dtype=torch.int16).view(torch.uint16)
+
+
+def alpha_of(rgba):
+    """the alpha channel, contiguous, through a signed view for uint16"""
+    s = rgba.view(torch.int16) if rgba.dtype == torch.uint16 else rgba
+    return s[..., 3].contiguous().view(rgba.dtype)
+
+
+def alternated(fns, launches, flush):
+    """per-launch CUDA-event times (ms) of each fn, launched in turn, L2 overwritten before each launch"""
+    for fn in fns:
+        fn()
+    torch.cuda.synchronize()
+    pairs = [[] for _ in fns]
+    for _ in range(launches):
+        for k, fn in enumerate(fns):
+            flush.add_(1)
+            a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            a.record()
+            fn()
+            b.record()
+            pairs[k].append((a, b))
+    torch.cuda.synchronize()
+    return [[a.elapsed_time(b) for a, b in p] for p in pairs]
+
+
+def tiled(args, dev):
+    import ctypes
+    res = {"gpu": gpu_info(), "hbm_peak": f"{HBM_PEAK_GBPS:.0f} GB/s (NVIDIA HGX B200 data sheet, per GPU)"}
+    lib = mwa_b200._abi.load()
+    parent = ctypes.CDLL(os.path.abspath(args.parent_lib))
+    for name in ("rgba8_ingest", "rgba8_egress", "rgba16_ingest", "rgba16_egress"):
+        fn = getattr(parent, name)
+        fn.restype, fn.argtypes = ctypes.c_int, getattr(lib, name).argtypes
+    flush = torch.zeros(128 * 2 ** 20, dtype=torch.float32, device=dev)            # 512 MiB
+    src = torch.ones(256 * 2 ** 20, dtype=torch.float32, device=dev)
+    dst = torch.empty_like(src)
+    ct = event_times(lambda: dst.copy_(src), args.launches, flush)
+    copy_gbps = 2 * src.numel() * 4 / (statistics.median(ct) * 1e-3) / 1e9
+    res["copy_1GiB"] = {"median_us": 1e3 * statistics.median(ct), "bytes": 2 * src.numel() * 4, "GBps": copy_gbps}
+    del src, dst
+
+    def run(fn, *a):
+        mwa_b200._abi.check(fn(*a, mwa_b200._abi.stream_handle()), fn.__name__)
+
+    # the untiled kernels, this build against the parent's, alternated
+    untiled = {}
+    for wl, (B, H, W) in {"bench_16x768x512": (bench.BATCH_PER_GPU, bench.IMG_H, bench.IMG_W),
+                          "1x3840x2160": (1, 2160, 3840)}.items():
+        for bits in (8, 16):
+            g = torch.Generator(device=dev).manual_seed(1)
+            rgba = random_samples((B, H, W, 4), bits, g, dev)
+            a = alpha_of(rgba)
+            Hp, Wp = padded(H), padded(W)
+            image = torch.empty(B, 3, Hp, Wp, device=dev)
+            alpha = torch.empty(B, 1, Hp, Wp, device=dev)
+            x_hat = torch.rand(B, 3, Hp, Wp, generator=g, device=dev)
+            out = torch.empty_like(rgba)
+            calls = {"ingest_rgba": lambda L: run(getattr(L, f"rgba{bits}_ingest"), rgba.data_ptr(), image.data_ptr(),
+                                                  alpha.data_ptr(), B, H, W, 4),
+                     "ingest_alpha": lambda L: run(getattr(L, f"rgba{bits}_ingest"), a.data_ptr(), None, alpha.data_ptr(),
+                                                   B, H, W, 1),
+                     "egress": lambda L: run(getattr(L, f"rgba{bits}_egress"), x_hat.data_ptr(), a.data_ptr(),
+                                             out.data_ptr(), B, H, W)}
+            for kname, call in calls.items():
+                this_t, parent_t = alternated([lambda: call(lib), lambda: call(parent)], args.launches, flush)
+                untiled[f"{wl}/rgba{bits}/{kname}"] = {
+                    k: {"median_us": 1e3 * statistics.median(t), "min_us": 1e3 * min(t), "max_us": 1e3 * max(t),
+                        "q1_us": 1e3 * statistics.quantiles(t, n=4)[0], "q3_us": 1e3 * statistics.quantiles(t, n=4)[2]}
+                    for k, t in (("this", this_t), ("parent", parent_t))}
+            del rgba, a, image, alpha, x_hat, out
+    res["untiled_kernels_this_vs_parent"] = untiled
+
+    # the tile kernels on one chunk of an 8192 x 8192 image
+    H = W = 8192
+    Th, Tw, ty, tx = mwa_b200.rgba8.tile_grid(H, W, 4096)
+    count = mwa_b200.rgba8.chunk_tiles(Th, Tw)
+    kern = {"H": H, "W": W, "tile": (Th, Tw), "grid": (ty, tx), "count": count}
+    px = count * Th * Tw                        # every pixel of these tiles lies in the image
+    for bits in (8, 16):
+        sb = bits // 8
+        g = torch.Generator(device=dev).manual_seed(2)
+        rgba = random_samples((1, H, W, 4), bits, g, dev)
+        a = alpha_of(rgba)
+        x_hat = torch.rand(count, 3, Th, Tw, generator=g, device=dev)
+        out = torch.empty_like(rgba)
+        r = mwa_b200.rgba8
+        for kname, fn, nbytes in (("ingest_rgba", lambda: r.ingest_tiles(rgba, (Th, Tw), 0, count), 4 * sb * px + 16 * px),
+                                  ("ingest_alpha", lambda: r.ingest_tiles(a[..., None], (Th, Tw), 0, count),
+                                   sb * px + 4 * px),
+                                  ("egress", lambda: r.egress_tiles(x_hat, a, out, 0), 12 * px + sb * px + 4 * sb * px)):
+            kern[f"rgba{bits}/{kname}"] = summary(event_times(fn, args.launches, flush), nbytes, copy_gbps)
+        del rgba, a, x_hat, out
+    res["tile_kernels_8192"] = kern
+    del flush
+
+    # the codec
+    torch.manual_seed(234)
+    net = mwa_b200.RGBACodec().eval().to(dev)
+    g = torch.Generator().manual_seed(3)
+
+    def picture(H, W):
+        """smooth colour in 16 x 16 blocks + noise, alpha 0 on ~25 % of the blocks (uint8 on the device)"""
+        small = torch.rand(1, 4, -(-H // 16), -(-W // 16), generator=g)
+        small[:, 3] = small[:, 3] * (small[:, 3] > 0.25)
+        big = torch.nn.functional.interpolate(small, scale_factor=16, mode="bilinear")[..., :H, :W]
+        big = (big + 0.03 * torch.randn(big.shape, generator=g)).clamp(0, 1)
+        big[:, 3] *= big[:, 3] > 0.2
+        return (big * 255).round().to(torch.uint8).permute(0, 2, 3, 1).contiguous().to(dev)
+
+    def measured(fn):
+        fn()
+        torch.cuda.synchronize()
+        torch.cuda.reset_peak_memory_stats()
+        med, runs, out = timed(fn, args.reps)
+        return {"median_ms": med, "runs_ms": runs, "max_memory_allocated_GB": torch.cuda.max_memory_allocated() / 1e9}, out
+
+    codec = {"model": "RGBACodec, random init under torch.manual_seed(234)",
+             "free_and_total_GB_at_start": [v / 1e9 for v in torch.cuda.mem_get_info()]}
+    t = picture(8192, 8192)
+    a8 = alpha_of(t)
+    with torch.no_grad():
+        for coder in ("host", "device"):
+            c, out = measured(lambda: net.compress_tiled(t, coder=coder))
+            d, rec = measured(lambda: net.decompress_tiled(out["strings"], out["shape"], a8))
+            n = len(out["strings"][0])
+            codec[f"1x8192x8192/{coder}"] = {
+                "grid": out["grid"], "shape": tuple(out["shape"]), "tiles": n,
+                "chunks": -(-n // mwa_b200.rgba8.chunk_tiles(64 * out["shape"][0], 64 * out["shape"][1])),
+                "bytes": sum(map(len, out["strings"][0])) + sum(map(len, out["strings"][1])),
+                "compress_tiled": c, "decompress_tiled": d,
+                "alpha_copied": bool(torch.equal(rec[..., 3], a8))}
+        del t, a8, rec
+        t = picture(4096, 4096)
+        a8 = alpha_of(t)
+        for coder in ("host", "device"):
+            for label, comp, decomp in (
+                    ("untiled", lambda: net.compress_rgba8(t, coder=coder),
+                     lambda o: net.decompress_rgba8(o["strings"], o["shape"], a8)),
+                    ("tile_2048", lambda: net.compress_tiled(t, 2048, coder=coder),
+                     lambda o: net.decompress_tiled(o["strings"], o["shape"], a8))):
+                c, out = measured(comp)
+                d, rec = measured(lambda: decomp(out))
+                err = (rec[..., :3].float() - t[..., :3].float()) * (a8[..., None] > 0)
+                codec[f"1x4096x4096/{coder}/{label}"] = {
+                    "tiles": len(out["strings"][0]),
+                    "bytes": sum(map(len, out["strings"][0])) + sum(map(len, out["strings"][1])),
+                    "compress": c, "decompress": d, "rgb_mse_opaque": float(err.square().sum() / (a8 > 0).sum() / 3)}
+    res["codec"] = codec
+    res["gpu_after"] = gpu_info()
+    os.makedirs(args.out, exist_ok=True)
+    with open(os.path.join(args.out, "rgba_tiled_time.json"), "w") as f:
+        json.dump(res, f, indent=1)
+    print(json.dumps(res))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--launches", type=int, default=50)
     ap.add_argument("--reps", type=int, default=5)
     ap.add_argument("--bits", type=int, choices=(8, 16), default=8, help="sample depth of the timed kernels")
-    ap.add_argument("--out", required=True, help="directory for rgba{bits}_time.json")
+    ap.add_argument("--tiled", action="store_true", help="measure the tiled path (rgba_tiled_time.json)")
+    ap.add_argument("--parent-lib", help="with --tiled: the previous commit's libmwa_b200.so, for the untiled kernels")
+    ap.add_argument("--out", required=True, help="directory for the JSON result")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         sys.exit("rgba8_time.py measures on a CUDA device; none found")
+    if args.tiled:
+        if not args.parent_lib:
+            sys.exit("--tiled needs --parent-lib")
+        return tiled(args, torch.device("cuda:0"))
     dev = torch.device("cuda:0")
     torch.backends.cudnn.allow_tf32 = False
     torch.backends.cuda.matmul.allow_tf32 = False
